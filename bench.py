@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          (N>1: launched under torch.distributed.run)
   python bench.py --impl reference ...                   (CPU arm: the oracle port of the reference, rank 0 only)
+  python bench.py ... --dump-outputs DIR                 (also writes the last timed step's outputs to DIR/*.npy)
 
 A "step" is one full differentiable render of the metric's workload -- SDFRenderer.render() of ONE 512x512 image (depth +
 normal + silhouette, 50-step 'recursive' march, buffer 5) with gradients enabled w.r.t. the 256-d latent, a scalar loss
@@ -219,6 +220,18 @@ def cpu_port_baseline(synth, lat_h, R_h, T_h):
                       "(best of a thread sweep)" % (Hc, Hc, 512 * 512 // (Hc * Hc), threads, os.cpu_count() or 1)}
 
 
+def dump_outputs(path, result):
+    """The result of the last timed step as its caller receives it -- the four full-image maps of render() and the
+    gradient w.r.t. the latent -- one float32 .npy per array (6.3 MB at 512x512), for comparing builds output by output.
+    The maps repeat bit for bit from run to run; the latent gradient is summed with float atomics and moved by ~4e-7
+    rel-L2 between runs on one B200."""
+    import numpy as np
+    (depth, normal, mask, min_sdf), latent_grad = result
+    os.makedirs(path, exist_ok=True)
+    for name, t in (("depth", depth), ("normal", normal), ("mask", mask), ("min_sdf", min_sdf), ("latent_grad", latent_grad)):
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def config_of(n_gpus, side=HW_BASE):
     return {"workload": "%dx%d render(): depth+normal+silhouette, single shape (geometric-init 8x512 DeepSDF, 256-d "
                         "latent), %d-step '%s' march, buffer %d, fwd + backward over the latent"
@@ -273,6 +286,7 @@ def main():
     ap.add_argument("--engine", default="auto")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the weak-scaling and config-5 extra measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -356,9 +370,16 @@ def main():
     gc.collect()
     gc.disable()   # no cyclic-GC pauses inside the timed regions (re-enabled below)
     l0 = lib.dist_launch_count()
+    last = [None]
+
+    def headline_step():
+        last[0] = step_device(lat_d, R_d, T_d)
     with ClockSampler(local_rank if not os.environ.get('BENCH_NO_SAMPLER') else -1) as clk:
-        ms, step_ms = timed(lambda: step_device(lat_d, R_d, T_d), args.steps, 0)
+        ms, step_ms = timed(headline_step, args.steps, 0)
     launches = lib.dist_launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last[0])
+    last[0] = None
     rows_f = int(ren.local.rows_evaluated.item())
     rows_g, rows_gc = [int(v) for v in ren.local.rows_grad.tolist()]     # full gradient rows (2F), mask-cache replays (F)
     tiles_1p, tiles_3p = [int(v) / args.steps for v in ren.local.tile_counters.tolist()]

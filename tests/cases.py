@@ -14,6 +14,12 @@ synth = importlib.import_module("dist-renderer_b200.synth")
 
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
 
+# The fp32 oracles' last bits depend on how many threads split their CPU GEMMs, and a march that starts inside the
+# shape turns such bits into visible differences.  The fixtures were written with this many threads; the tests and
+# oracle/make_golden.py use the same count on any host, whatever its number of cores.
+CPU_THREADS = 8
+torch.set_num_threads(CPU_THREADS)
+
 # name -> recipe.  cam: ('front', dist) or ('lookat', az, el, dist, focal_scale)
 CASES = {
     "c1_recursive_64": dict(decoder="B", hw=(64, 64), cam=("front", 1.6), march_step=50, buffer_size=5,
@@ -118,6 +124,43 @@ def color_case():
     g = torch.Generator().manual_seed(13)
     color_code = 0.1 * torch.randn(1, 8, generator=g)
     return hw, K, R, T, color_code, torch.tensor([[0.5, 1.0, -3.0]]), torch.tensor([0.8])
+
+
+def color_lighting(lights, energies):
+    """The lighting arguments of SDFRenderer_color.render compared with the reference: none, locations, both."""
+    return [dict(), dict(lighting_locations=lights), dict(lighting_locations=lights, lighting_energies=energies)]
+
+
+def loss_case():
+    """The single-view loss (loss_single.py:7-57) on a 40x40 view; the renderer runs a 60-step march with buffer 3."""
+    hw = (40, 40)
+    return (hw, synth.intrinsic(*hw)) + synth.lookat_camera(30.0, 20.0, 1.8)
+
+
+# depth maps fed to depth2normal (renderer.py:972-975), degenerate sizes included
+D2N_SHAPES = [(7, 9), (40, 33), (3, 3), (2, 5), (1, 1)]
+
+SMALL_SPEC = dict(dims=[64] * 8, dropout=list(range(8)), dropout_prob=0.2, norm_layers=list(range(8)), latent_in=[4],
+                  xyz_in_all=False, use_tanh=False, latent_dropout=False, weight_norm=True)
+
+
+def write_experiment(root, make_decoder):
+    """An experiment directory in the upstream DeepSDF layout: specs.json, an SDF checkpoint saved from a DataParallel
+    wrapper (keys prefixed `module.`) and a colour checkpoint saved without the prefix (decoder_utils.py:33-41).
+    Returns the colour experiment's directory."""
+    import json
+    json.dump({"NetworkArch": "deep_sdf_decoder", "CodeLength": 16, "NetworkSpecs": SMALL_SPEC},
+              open(os.path.join(root, "specs.json"), "w"))
+    col = os.path.join(root, "color")
+    os.makedirs(os.path.join(root, "ModelParameters"))
+    os.makedirs(os.path.join(col, "ModelParameters"))
+    torch.manual_seed(0)
+    sdf = torch.nn.DataParallel(make_decoder(16, **SMALL_SPEC))
+    torch.save({"epoch": 1, "model_state_dict": sdf.state_dict()}, os.path.join(root, "ModelParameters", "latest.pth"))
+    cspec = dict(SMALL_SPEC, dims=[64, 64, 64, 72, 64, 64, 64, 64])
+    torch.save({"epoch": 1, "model_state_dict": make_decoder(24, last_dim=3, **cspec).state_dict()},
+               os.path.join(col, "ModelParameters", "latest.pth"))
+    return col
 
 
 def warp_case():

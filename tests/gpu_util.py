@@ -58,6 +58,12 @@ def run_oracle(cs, grads=True, dec=None, dtype=torch.float32):
     return [o.detach() for o in out], g
 
 
+def at_pixels(maps, pix):
+    """(depth, normal, mask, min_sdf) maps restricted to the flat pixel indices `pix` (a fixture's stored sample)."""
+    idx = torch.as_tensor(pix, dtype=torch.long)
+    return [m.reshape(-1, *m.shape[2:])[idx] for m in maps]
+
+
 def normal_error(n_a, n_b, mask, outlier_frac=0.005, outlier_thresh=1e-3):
     """rel-L2 of the normal map on `mask` after dropping at most outlier_frac pixels whose per-pixel error exceeds
     outlier_thresh (ReLU-boundary flips: the fp32 reference vs its own fp64 twin shows the same, SURVEY.md H2).

@@ -1,6 +1,6 @@
 """CPU: the marching-cubes case table (product side, dist-renderer_b200/mc_tables.py) against the oracle's independent
-per-cube tracing, the oracle against properties of analytic shapes, and the chamfer oracle against the reference's own
-eval_func.py (scipy is installed; /root/reference only in the build container) and its committed outputs."""
+per-cube tracing, the oracle against properties of analytic shapes, and the chamfer oracle against the outputs of the
+reference's own eval_func.py (tests/golden/chamfer.npz)."""
 import importlib
 import os
 
@@ -10,7 +10,6 @@ import pytest
 import cases  # noqa: F401  (puts the repo root on sys.path)
 import mesh_cases
 from oracle import mesh_oracle as O
-from oracle import ref_shim
 
 mc_tables = importlib.import_module("dist-renderer_b200.mc_tables")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -107,13 +106,13 @@ def _chamfer_inputs():
     return a, b
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 def test_chamfer_oracle_matches_reference():
-    EF = ref_shim.load_eval_func()
+    """Bit for bit: the oracle's float results equal the reference's."""
+    g = np.load(GOLD)
     a, b = _chamfer_inputs()
-    assert O.compute_chamfer_distance(a, b) == EF.compute_chamfer_distance(a, b)
-    assert O.compute_chamfer_distance(a, b, False) == EF.compute_chamfer_distance(a, b, use_square_dist=False)
-    assert O.compute_chamfer_distance_separate(a, b) == tuple(float(x) for x in EF.compute_chamfer_distance_separate(a, b))
+    assert O.compute_chamfer_distance(a, b) == float(g["sq"])
+    assert O.compute_chamfer_distance(a, b, False) == float(g["lin"])
+    assert O.compute_chamfer_distance_separate(a, b) == tuple(float(x) for x in g["sep"])
 
 
 def test_chamfer_oracle_matches_golden():

@@ -1,15 +1,12 @@
-"""CPU: pin oracle/sdf_oracle.py against (a) golden fixtures written from the real reference and
-(b) the real reference itself where /root/reference is present (the build container)."""
+"""CPU: pin the oracles (oracle/*.py) against golden fixtures that hold outputs of the real reference
+(tests/golden, written by oracle/make_golden.py)."""
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
 import cases
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-from oracle import ref_shim
 from oracle.sdf_oracle import OracleSDFRenderer, decode_sdf, decode_sdf_gradient
 
 
@@ -90,45 +87,43 @@ def test_oracle_earlybreak_padding_render_depth(name):
         assert _rel(g.numpy(), gold[key]) < 1e-4, key
 
 
-def _loss_setup(hw=(40, 40)):
-    K, (R, T) = cases.synth.intrinsic(*hw), cases.synth.lookat_camera(30.0, 20.0, 1.8)
-    ora = OracleSDFRenderer(cases.decoder("B"), K, img_hw=hw, march_step=60, buffer_size=3)
-    gt = ora.render(cases.synth.make_latent(seed=2), R, T, no_grad=True)
-    gt_pack = {"depth": gt[0].detach(), "normal": gt[1].detach(), "silhouette": gt[2].detach()}
-    return hw, K, R, T, ora, gt_pack
+def _golden(name):
+    return np.load(os.path.join(cases.GOLDEN_DIR, name + ".npz"))
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_loss_oracle_matches_live_reference():
-    """oracle/loss_oracle.py == the reference's compute_all_loss (loss_single.py:7-57) on the reference's renderer:
-    every term of the loss pack, the weighted total and its gradient w.r.t. the shape code."""
+    """oracle/loss_oracle.py == the reference's compute_all_loss (loss_single.py:7-57) on the reference's renderer
+    (tests/golden/loss_40.npz, with the ground-truth maps it was given): every term of the loss pack, the weighted total
+    and its gradient w.r.t. the shape code."""
     from oracle import loss_oracle
-    import make_golden
-    hw, K, R, T, ora, gt_pack = _loss_setup()
-    Rmod, _, _ = ref_shim.load()
-    ref_loss = ref_shim.load_loss_single()
-    ren = Rmod.SDFRenderer(make_golden.ref_decoder(cases.decoder("B")), K, img_hw=hw, march_step=60, buffer_size=3, use_gpu=False)
-    ext = torch.cat([R, T[:, None]], 1)
-    l_r = cases.synth.make_latent().requires_grad_(True)
-    pack_r, _ = ref_loss(ren, l_r, ext, gt_pack, ray_marching_type='recursive')
-    loss_oracle.total(pack_r).backward()
+    gold = _golden("loss_40")
+    hw, K, R, T = cases.loss_case()
+    ora = OracleSDFRenderer(cases.decoder("B"), K, img_hw=hw, march_step=60, buffer_size=3)
+    gt_pack = {k: torch.from_numpy(gold["gt_" + k]) for k in ("depth", "normal", "silhouette")}
     l_o = cases.synth.make_latent().requires_grad_(True)
-    pack_o = loss_oracle.compute_all_loss(ora, l_o, ext, gt_pack, ray_marching_type='recursive')
+    pack_o = loss_oracle.compute_all_loss(ora, l_o, torch.cat([R, T[:, None]], 1), gt_pack, ray_marching_type='recursive')
     loss_oracle.total(pack_o).backward()
     for k in ("mask_gt", "mask_out", "depth", "normal", "l2reg"):
-        assert abs(float(pack_o[k]) - float(pack_r[k])) <= 1e-6 * max(1.0, abs(float(pack_r[k]))), k
-    assert float(pack_r["depth"]) > 0 and float(pack_r["normal"]) < 0
-    assert _rel(l_o.grad.numpy(), l_r.grad.numpy()) < 1e-5
+        ref = float(gold["pack_" + k])
+        assert abs(float(pack_o[k]) - ref) <= 1e-6 * max(1.0, abs(ref)), k
+    assert float(gold["pack_depth"]) > 0 and float(gold["pack_normal"]) < 0
+    assert _rel(l_o.grad.numpy(), gold["g_latent"]) < 1e-5
 
 
 def test_big_fixtures_present_and_consistent():
     """The BASELINE-size fixtures (cases.BIG_CASES; written by `oracle/make_golden.py --big` from the real reference)
-    are too slow to re-render in the CPU suite: check they exist, match the seeded decoder and carry their fp64 floor."""
+    are too slow to re-render in the CPU suite: check they exist, match the seeded decoder and carry their fp64 floor.
+    Above 256x256 pixels a fixture holds the maps at a sample of distinct pixels (`pix`, flat indices) and the mask whole."""
     for name, cs in cases.BIG_CASES.items():
         gold = np.load(os.path.join(cases.GOLDEN_DIR, "big_" + name + ".npz"))
         assert abs(cases.weights_checksum(cases.decoder(cs["decoder"])) - float(gold["weights_checksum"])) < 1e-6
-        assert gold["depth"].shape == cs["hw"] and gold["normal"].shape == cs["hw"] + (3,)
-        assert gold["mask"].dtype == np.uint8 and 0.05 < gold["mask"].mean() < 0.6
+        shape = cs["hw"]
+        if cs["hw"][0] * cs["hw"][1] > 256 * 256:
+            pix = gold["pix"]
+            assert np.all(np.diff(pix) > 0) and 0 <= pix[0] and pix[-1] < cs["hw"][0] * cs["hw"][1]
+            shape = pix.shape
+        assert gold["depth"].shape == shape and gold["normal"].shape == shape + (3,) and gold["min_sdf"].shape == shape
+        assert gold["mask"].shape == cs["hw"] and gold["mask"].dtype == np.uint8 and 0.05 < gold["mask"].mean() < 0.6
         floor = dict(zip(gold["floor_keys"].tolist(), gold["floor_vals"].tolist()))
         assert floor["depth"] < 1e-5 and floor["xor"] <= 0.0005 * gold["mask"].size, floor
 
@@ -142,104 +137,69 @@ def test_oracle_decoder_points_golden():
     assert _rel(decode_sdf_gradient(dec, lat, p).detach().numpy(), gold["grad"]) < 1e-5
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 @pytest.mark.parametrize("name", ["trivial_40", "inside_32"])
 def test_oracle_matches_live_reference(name):
+    """The reference's render() without gradients (tests/golden/nograd_*.npz)."""
     cs = cases.CASES[name]
-    Rmod, _, RefDecoder = ref_shim.load()
-    dec = cases.decoder(cs["decoder"])
-    ref = RefDecoder(dec.latent_size, **cases.synth.STANDARD_SPEC).eval()
-    ref.load_state_dict(dec.state_dict())
-    K, R, T = cases.camera(cs["cam"], cs["hw"])
-    ren = Rmod.SDFRenderer(ref, K, img_hw=cs["hw"], march_step=cs["march_step"], buffer_size=cs["buffer_size"],
-                           use_gpu=False)
-    a = ren.render(cases.synth.make_latent(), R, T, ray_marching_type=cs["kind"], no_grad=True)
+    gold = _golden("nograd_" + name)
+    a = [torch.from_numpy(gold[k]) for k in ("depth", "normal", "mask", "min_sdf")]
     b, _ = _run_oracle(cs)
     assert int((a[2] != b[2]).sum()) == 0
     for i in (0, 1, 3):
         assert _rel(b[i].detach(), a[i]) < 1e-6
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_depth2normal_matches_live_reference():
     """use_depth2normal (renderer.py:972-975): the oracle's restatement and the product's host-side mirror
-    (device-agnostic PyTorch, so checked here on CPU) against the reference's own function, bit for bit, including the
-    in-place zeroing of the background of the depth map; then the whole render() branch, oracle vs reference."""
+    (device-agnostic PyTorch, so checked here on CPU) against the reference's own function (its outputs on the same
+    seeded maps in tests/golden/depth2normal.npz), bit for bit, including the in-place zeroing of the background of the
+    depth map; then the whole render() branch, oracle vs reference."""
     import importlib
-    import sys
-    import numpy as np
     from oracle.sdf_oracle import depth2normal as d2n_oracle
-    Rmod, _, RefDecoder = ref_shim.load()
-    d2n_ref = sys.modules["core.utils.render_utils"].depth2normal
+    gold = _golden("depth2normal")
     d2n_prod = importlib.import_module("dist-renderer_b200.render_utils").depth2normal
     g = torch.Generator().manual_seed(3)
-    for (h, w) in [(7, 9), (40, 33), (3, 3), (2, 5), (1, 1)]:
+    for i, (h, w) in enumerate(cases.D2N_SHAPES):
         d = torch.rand(h, w, generator=g) * 2 + 0.5
         d[torch.rand(h, w, generator=g) < 0.3] = 1e11
         d[0, 0] = 0.0
         fx, fy = np.float32(57.6), np.float32(50.0)
-        da, db, dc = d.clone(), d.clone(), d.clone()
-        a, b, c = d2n_ref(da, fx, fy), d2n_oracle(db, fx, fy), d2n_prod(dc, fx, fy)
+        da, db, dc = torch.from_numpy(gold["depth_%d" % i]), d.clone(), d.clone()
+        a, b, c = torch.from_numpy(gold["normal_%d" % i]), d2n_oracle(db, fx, fy), d2n_prod(dc, fx, fy)
         assert torch.equal(a, b) and torch.equal(a, c)
         assert torch.equal(da, db) and torch.equal(da, dc) and float(da[0, 0]) == 0.0
     # gradients w.r.t. the depth agree (the product forms the differences before scattering: last-bit differences)
     d = torch.rand(12, 12, generator=g) + 0.5
     d[2:4, 3] = 1e11
     wgt = torch.randn(12, 12, 3, generator=g)
-    grads = []
-    for fn in (d2n_ref, d2n_oracle, d2n_prod):
+    grads = [torch.from_numpy(gold["grad"])]
+    for fn in (d2n_oracle, d2n_prod):
         x = d.clone().requires_grad_(True)
         (fn(x * 1.0, np.float32(30.0)) * wgt).sum().backward()
         grads.append(x.grad)
     assert torch.equal(grads[0], grads[1]) and _rel(grads[2], grads[0]) < 1e-6
     # the render() branch
     cs = cases.CASES["trivial_40"]
-    dec = cases.decoder(cs["decoder"])
-    ref = RefDecoder(dec.latent_size, **cases.synth.STANDARD_SPEC).eval()
-    ref.load_state_dict(dec.state_dict())
     K, R, T = cases.camera(cs["cam"], cs["hw"])
     kw = dict(img_hw=cs["hw"], march_step=cs["march_step"], buffer_size=cs["buffer_size"], use_depth2normal=True)
-    a = Rmod.SDFRenderer(ref, K, use_gpu=False, **kw).render(cases.synth.make_latent(), R, T,
-                                                            ray_marching_type="recursive", no_grad=True)
-    b = OracleSDFRenderer(dec, K, **kw).render(cases.synth.make_latent(), R, T, ray_marching_type="recursive",
-                                               no_grad=True)
+    a = [torch.from_numpy(gold["render_" + k]) for k in ("depth", "normal", "mask", "min_sdf")]
+    b = OracleSDFRenderer(cases.decoder(cs["decoder"]), K, **kw).render(cases.synth.make_latent(), R, T,
+                                                                         ray_marching_type="recursive", no_grad=True)
     for x, y in zip(a, b):
         assert torch.equal(x, y)
     assert float(a[0].min()) == 0.0 and float(a[0].max()) < 1e5      # background of the returned depth is 0, not 1e11
 
 
-_SMALL_SPEC = dict(dims=[64] * 8, dropout=list(range(8)), dropout_prob=0.2, norm_layers=list(range(8)), latent_in=[4],
-                   xyz_in_all=False, use_tanh=False, latent_dropout=False, weight_norm=True)
-
-
-def _write_experiment(root, make_decoder):
-    """An experiment directory in the upstream DeepSDF layout: specs.json, an SDF checkpoint saved from a DataParallel
-    wrapper (keys prefixed `module.`) and a colour checkpoint saved without the prefix (decoder_utils.py:33-41)."""
-    import json
-    import os
-    json.dump({"NetworkArch": "deep_sdf_decoder", "CodeLength": 16, "NetworkSpecs": _SMALL_SPEC},
-              open(os.path.join(root, "specs.json"), "w"))
-    col = os.path.join(root, "color")
-    os.makedirs(os.path.join(root, "ModelParameters"))
-    os.makedirs(os.path.join(col, "ModelParameters"))
-    torch.manual_seed(0)
-    sdf = torch.nn.DataParallel(make_decoder(16, **_SMALL_SPEC))
-    torch.save({"epoch": 1, "model_state_dict": sdf.state_dict()}, os.path.join(root, "ModelParameters", "latest.pth"))
-    cspec = dict(_SMALL_SPEC, dims=[64, 64, 64, 72, 64, 64, 64, 64])
-    torch.save({"epoch": 1, "model_state_dict": make_decoder(24, last_dim=3, **cspec).state_dict()},
-               os.path.join(col, "ModelParameters", "latest.pth"))
-    return col
-
-
 def test_load_decoder_roundtrip(tmp_path):
     """load_decoder (decoder_utils.py:7-51): SDF and colour decoders, DataParallel wrapper by default."""
-    col = _write_experiment(str(tmp_path), cases.pkg.Decoder)
+    col = cases.write_experiment(str(tmp_path), cases.pkg.Decoder)
     wrapped = cases.pkg.load_decoder(str(tmp_path), "latest")
     assert isinstance(wrapped, torch.nn.DataParallel) and wrapped.module.latent_size == 16
     bare = cases.pkg.load_decoder(str(tmp_path), "latest", parallel=False)
     x = torch.randn(9, 19)
-    assert torch.equal(wrapped.module.eval().inference(x), bare.eval().inference(x))
-    colour = cases.pkg.load_decoder(str(tmp_path), "latest", color_size=8, experiment_directory_color=col).module.eval()
+    # DataParallel moves the module to cuda:0 where a GPU is present: compared on the host
+    assert torch.equal(wrapped.module.eval().cpu().inference(x), bare.eval().inference(x))
+    colour = cases.pkg.load_decoder(str(tmp_path), "latest", color_size=8, experiment_directory_color=col).module.eval().cpu()
     assert colour.latent_size == 24 and colour.lin3.weight_v.shape[0] == 72 - 27 and colour.lin8.out_features == 3
     rgb = colour.inference(torch.cat([torch.randn(1, 16).expand(70, -1), torch.randn(1, 8).expand(70, -1), torch.randn(70, 3)], 1))
     assert rgb.shape == (70, 3) and float(rgb.abs().max()) <= 1.0
@@ -249,20 +209,21 @@ def test_load_decoder_roundtrip(tmp_path):
         cases.pkg.load_decoder(str(tmp_path / "nowhere"))
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_load_decoder_and_decode_color_match_live_reference(tmp_path):
-    _, DU, RefDecoder = ref_shim.load()
-    col = _write_experiment(str(tmp_path), RefDecoder)
-    a = DU.load_decoder(str(tmp_path), "latest").module.eval()
-    b = cases.pkg.load_decoder(str(tmp_path), "latest").module.eval()
-    x = torch.randn(50, 19)
-    assert torch.equal(a.inference(x), b.inference(x))
-    ac = DU.load_decoder(str(tmp_path), "latest", color_size=8, experiment_directory_color=col).module.eval()
-    bc = cases.pkg.load_decoder(str(tmp_path), "latest", color_size=8, experiment_directory_color=col).module.eval()
-    pts, sc, cc = torch.randn(70, 3), torch.randn(1, 16), torch.randn(1, 8)
+    """The reference's load_decoder and decode_color on the same experiment (its outputs and weight checksums in
+    tests/golden/load_decoder.npz; the reference's Decoder writes the same weights as the product's)."""
+    gold = _golden("load_decoder")
+    col = cases.write_experiment(str(tmp_path), cases.pkg.Decoder)
+    b = cases.pkg.load_decoder(str(tmp_path), "latest").module.eval().cpu()
+    assert cases.weights_checksum(b) == float(gold["sdf_checksum"])
+    x = torch.from_numpy(gold["x"])
+    assert torch.equal(torch.from_numpy(gold["sdf"]), b.inference(x))
+    bc = cases.pkg.load_decoder(str(tmp_path), "latest", color_size=8, experiment_directory_color=col).module.eval().cpu()
+    assert cases.weights_checksum(bc) == float(gold["color_checksum"])
+    pts, sc, cc = (torch.from_numpy(gold[k]) for k in ("pts", "shape_code", "color_code"))
     # the reference's decode_color rows are [shape code | colour code | xyz] (decoder_utils.py:103): same module outputs
     rows = torch.cat([sc.expand(70, -1), cc.expand(70, -1), pts], 1)
-    assert _rel(DU.decode_color(ac, cc, sc, pts, MAX_POINTS=32).detach(), bc.inference(rows).detach()) < 1e-6   # (chunked GEMMs)
+    assert _rel(torch.from_numpy(gold["rgb"]), bc.inference(rows).detach()) < 1e-6   # (chunked GEMMs)
 
 
 def _color_setup():
@@ -291,72 +252,56 @@ def test_color_oracle_matches_golden():
     assert _rel(plain[2], torch.from_numpy(gold["color_unlit"])) < 1e-6
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_color_oracle_matches_live_reference():
-    """Bit-for-bit against renderer_rgb.py run through the shim: outputs, and gradients w.r.t. both codes."""
-    _, _, RefDecoder = ref_shim.load()
-    Color = ref_shim.load_color()
+    """Bit-for-bit against renderer_rgb.py (its outputs in tests/golden/color_lighting_24.npz): outputs under each
+    lighting argument, and gradients w.r.t. both codes."""
+    gold = _golden("color_lighting_24")
     ora, col, (hw, K, R, T, cc, lights, energies) = _color_setup()
-    dec = cases.decoder("B")
-    ref_sdf = RefDecoder(dec.latent_size, **cases.synth.STANDARD_SPEC).eval()
-    ref_sdf.load_state_dict(dec.state_dict())
-    ref_col = RefDecoder(col.latent_size, last_dim=3, **dict(cases.synth.STANDARD_SPEC, dims=list(col.dims[1:-1]))).eval()
-    ref_col.load_state_dict(col.state_dict())
-    ren = Color(ref_sdf, ref_col, K, img_hw=hw, use_gpu=False)
     lat = cases.synth.make_latent()
-    for kw in (dict(), dict(lighting_locations=lights), dict(lighting_locations=lights, lighting_energies=energies)):
-        a, b = ren.render(cc, lat, R, T, no_grad=True, **kw), ora.render(cc, lat, R, T, no_grad=True, **kw)
-        assert all(torch.equal(x, y) for x, y in zip(a, b))
-    grads = []
-    for r in (ren, ora):
-        l, c = lat.clone().requires_grad_(True), cc.clone().requires_grad_(True)
-        o = r.render(c, l, R, T, lighting_locations=lights)
-        (o[2].sum() + o[0][o[3].bool()].sum()).backward()
-        grads.append((l.grad, c.grad))
-    assert torch.equal(grads[0][0], grads[1][0]) and torch.equal(grads[0][1], grads[1][1])
+    for i, kw in enumerate(cases.color_lighting(lights, energies)):
+        b = ora.render(cc, lat, R, T, no_grad=True, **kw)
+        assert all(torch.equal(torch.from_numpy(gold["out_%d_%d" % (i, j)]), y) for j, y in enumerate(b))
+    l, c = lat.clone().requires_grad_(True), cc.clone().requires_grad_(True)
+    o = ora.render(c, l, R, T, lighting_locations=lights)
+    (o[2].sum() + o[0][o[3].bool()].sum()).backward()
+    assert torch.equal(torch.from_numpy(gold["g_latent"]), l.grad) and torch.equal(torch.from_numpy(gold["g_color"]), c.grad)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_deepsdf_sampler_host_logic_matches_live_reference(monkeypatch):
     """SDFRenderer_deepsdf.get_samples / get_freespace_samples (renderer_deepsdf.py:14-65).  The product methods are
     device-agnostic host code around decode_sdf; here they run on CPU -- on a renderer object whose constructor (which
     insists on a CUDA decoder) is bypassed and whose decoder calls are routed to the oracle's decode_sdf -- against the
-    reference class executed through the shim, bit for bit, including the random draws under a common seed."""
+    reference class's outputs on the same depth and normal maps (tests/golden/deepsdf_samples_24.npz), bit for bit,
+    including the random draws under a common seed."""
     import importlib
-    import numpy as np
     from oracle.sdf_oracle import decode_sdf as oracle_decode
-    Deep = ref_shim.load_deepsdf()
-    _, _, RefDecoder = ref_shim.load()
+    gold = _golden("deepsdf_samples_24")
     mod = importlib.import_module("dist-renderer_b200.renderer_deepsdf")
     monkeypatch.setattr(mod.functional, "decode_sdf",
                         lambda dec, lat, pts, clamp_dist=0.1, **kw: oracle_decode(dec, lat, pts, clamp_dist=clamp_dist))
     hw = (24, 24)
     K, R, T = cases.camera(("front", 1.6), hw)
     dec = cases.decoder("B")
-    ref_dec = RefDecoder(dec.latent_size, **cases.synth.STANDARD_SPEC).eval()
-    ref_dec.load_state_dict(dec.state_dict())
     lat = cases.synth.make_latent()
-    depth, normal, _, _ = OracleSDFRenderer(dec, K, img_hw=hw).render(lat, R, T, ray_marching_type="recursive",
-                                                                       no_grad=True)
+    depth, normal = torch.from_numpy(gold["depth"]), torch.from_numpy(gold["normal"])
     RT = torch.cat([R, T[:, None]], 1)
-    ref = Deep(ref_dec, K, img_hw=hw, use_gpu=False)
     prod = object.__new__(mod.SDFRenderer_deepsdf)            # no CUDA here: set what the camera helpers read
     prod.decoder, prod.device, prod.img_hw, prod.rows, prod.Pv = dec, torch.device("cpu"), hw, (0, 1, hw[0], 1), hw[0] * hw[1]
     prod.K_inv = torch.from_numpy(np.linalg.inv(K)).float()
     prod.transform_matrix = torch.tensor([[1., 0., 0.], [0., 0., -1.], [0., 1., 0.]])
     prod._homo_calib = prod._calib_map = None
-    a = ref.get_samples(lat, RT, depth.clone(), normal.clone(), use_rand=False)
+    a = (torch.from_numpy(gold["fixed_0"]), torch.from_numpy(gold["fixed_1"]))
     b = prod.get_samples(lat, RT, depth.clone(), normal.clone(), use_rand=False)
     assert a[0].numel() == int(((depth < 1e5) & (depth > 0)).sum()) > 50
     assert torch.equal(a[0], b[0]) and torch.equal(a[1], b[1])
     assert float(a[0].detach().abs().max()) < 0.05 and float(a[1].detach().abs().max()) < 0.05   # near zero: the samples straddle the surface
-    for fn, args in (("get_samples", (depth.clone(), normal.clone())), ("get_freespace_samples", (depth.clone(),))):
-        torch.manual_seed(21)
-        x = getattr(ref, fn)(lat, RT, *args)
+    for fn, args, keys in (("get_samples", (depth.clone(), normal.clone()), ("random_0", "random_1")),
+                           ("get_freespace_samples", (depth.clone(),), ("freespace",))):
+        x = tuple(torch.from_numpy(gold[k]) for k in keys)
         torch.manual_seed(21)
         y = getattr(prod, fn)(lat, RT, *args)
-        x, y = (x, y) if isinstance(x, tuple) else ((x,), (y,))
-        assert all(torch.equal(p, q) for p, q in zip(x, y))
+        y = y if isinstance(y, tuple) else (y,)
+        assert len(x) == len(y) and all(torch.equal(p, q) for p, q in zip(x, y))
     torch.manual_seed(3)
     free = prod.get_freespace_samples(lat, RT, depth.clone(), number=3)
     assert free.numel() == 3 * a[0].numel() and float(free.min()) > -0.05       # in front of the surface the sdf is positive
@@ -400,40 +345,25 @@ def test_warp_oracle_matches_golden():
     assert _rel(out[6].detach().numpy(), gold["depth1"]) < 1e-6
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_warp_oracle_matches_live_reference():
+    """The reference's render_warp loss and first-view normals (tests/golden/warp_40.npz) at the tight bar."""
     from oracle.warp_oracle import OracleWarpRenderer
-    Warp = ref_shim.load_warp()
-    _, _, RefDecoder = ref_shim.load()
-    dec = cases.decoder("B")
-    ref = RefDecoder(dec.latent_size, **cases.synth.STANDARD_SPEC).eval()
-    ref.load_state_dict(dec.state_dict())
+    gold = _golden("warp_40")
     hw, K, (R1, T1), (R2, T2), img1, img2 = cases.warp_case()
-    a = Warp(ref, K, img_hw=hw, use_gpu=False).render_warp(cases.synth.make_latent(), R1, T1, R2, T2, img1, img2)
-    b = OracleWarpRenderer(dec, K, img_hw=hw).render_warp(cases.synth.make_latent(), R1, T1, R2, T2, img1, img2)
-    assert abs(float(a[0]) - float(b[0])) < 1e-7
-    assert _rel(b[5].detach(), a[7].detach()) < 1e-6
+    b = OracleWarpRenderer(cases.decoder("B"), K, img_hw=hw).render_warp(cases.synth.make_latent(), R1, T1, R2, T2, img1, img2)
+    assert abs(float(gold["loss"]) - float(b[0])) < 1e-7
+    assert _rel(b[5].detach(), torch.from_numpy(gold["normal1"])) < 1e-6
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
 def test_grid_oracle_matches_live_reference():
-    """oracle/grid_oracle.py vs the reference's create_mesh.py sampling functions (next-2)."""
+    """oracle/grid_oracle.py vs the reference's create_mesh.py sampling functions (next-2): the sample coordinates and
+    the sparse-evaluated grid, bit for bit (sha256 of the reference's arrays in tests/golden/grid_64.npz)."""
+    import hashlib
     from oracle import grid_oracle
-    CM = ref_shim.load_create_mesh()
-    _, _, RefDecoder = ref_shim.load()
-    dec = cases.decoder("B")
-    ref = RefDecoder(dec.latent_size, **cases.synth.STANDARD_SPEC).eval()
-    ref.load_state_dict(dec.state_dict())
-    lat = cases.synth.make_latent()
+    gold = _golden("grid_64")
+    digest = lambda t: hashlib.sha256(np.ascontiguousarray(t.numpy()).tobytes()).hexdigest()
     N = 64          # 1.5 coarse voxels = 0.097 < the 0.1 clamp: the near/far classification becomes selective
-    vs, vsh = 2.0 / (N - 1), 2.0 / (N / 2 - 1)
-    assert torch.equal(CM.get_samples(N, [-1, -1, -1], vs, transform=True)[:, :3],
-                       grid_oracle.get_samples(N, [-1, -1, -1], vs, True))
-    sh = CM.get_samples(int(N / 2), [-1, -1, -1], vsh)
-    up = CM.upsample_cubic(CM.infer_samples(ref, lat, sh), int(N / 2), N)
-    pos, neg, val = CM.check_valid(up, vsh)
-    s = CM.get_samples(N, [-1, -1, -1], vs)
-    s[pos, 3], s[neg, 3] = 0.1, -0.1
-    s[val, 3] = CM.infer_samples(ref, lat, s[val, :])
-    og, n = grid_oracle.grid_speedup(dec, lat, N)
-    assert torch.equal(s[:, 3].reshape(N, N, N), og) and 0 < n < N ** 3
+    vs = 2.0 / (N - 1)
+    assert digest(grid_oracle.get_samples(N, [-1, -1, -1], vs, True)) == str(gold["coords_sha256"])
+    og, n = grid_oracle.grid_speedup(cases.decoder("B"), cases.synth.make_latent(), N)
+    assert digest(og) == str(gold["grid_sha256"]) and 0 < n < N ** 3
