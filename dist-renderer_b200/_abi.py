@@ -29,7 +29,7 @@ class Net(C.Structure):
                 ("Wt", C.c_void_p * MAX_LAYERS), ("W", C.c_void_p * MAX_LAYERS), ("bias", C.c_void_p * MAX_LAYERS),
                 ("Wz0", C.c_void_p), ("b0", C.c_void_p), ("Wzl", C.c_void_p), ("bl", C.c_void_p),
                 ("tc_blob", C.c_void_p), ("tc_scale", C.c_void_p), ("tc_blob_bytes", C.c_int64),
-                ("tc_bias", C.c_void_p * MAX_LAYERS)]
+                ("tc_bias", C.c_void_p * MAX_LAYERS), ("n_codes", C.c_int32), ("row_code", C.c_void_p)]
 
 
 class Camera(C.Structure):

@@ -64,6 +64,7 @@ int mlp_launch(const dist_net_t* net, const NetDev& nd, int engine, int mode, co
       if (a.grad) a2.grad = a.grad + 3 * o;
       if (a.coef) a2.coef = a.coef + o;
       if (a.use_clamp) a2.use_clamp = a.use_clamp + o;
+      if (a.row_code) a2.row_code = a.row_code + o;
       rc = mlp_simt_launch(nd, mode, a2, stream);
     }
   }
@@ -89,16 +90,20 @@ int make_netdev(const dist_net_t* net, NetDev* out) {
     out->K[l] = net->K[l]; out->N[l] = net->N[l];
     out->Wt[l] = net->Wt[l]; out->W[l] = net->W[l]; out->bias[l] = net->bias[l];
   }
+  DIST_REQUIRE(net->n_codes >= 0, "net: n_codes %d < 0", net->n_codes);
+  out->n_codes = net->n_codes > 1 ? net->n_codes : 1;
   DIST_REQUIRE(net->N[net->n_layers - 1] == 1, "net: last layer must have one output (got %d)", net->N[net->n_layers - 1]);
   return DIST_OK;
 }
 
 namespace {
-// out[n] = b[n] + Wz[n,:] . latent     one warp per output row
+// out[n] = b[n] + Wz[n,:] . latent     one warp per output row; code c = blockIdx.y reads latent[c][:], writes out[c][:]
 __global__ void k_fold(const float* __restrict__ Wz, const float* __restrict__ b, const float* __restrict__ latent,
                        int N, int Lz, float* __restrict__ out, int Npad) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= Npad) return;
+  latent += (size_t)blockIdx.y * Lz;
+  out += (size_t)blockIdx.y * Npad;
   float s = 0.f;
   if (warp < N) {
     for (int k = lane; k < Lz; k += 32) s = fmaf(Wz[(size_t)warp * Lz + k], latent[k], s);
@@ -106,6 +111,13 @@ __global__ void k_fold(const float* __restrict__ Wz, const float* __restrict__ b
     s += b[warp];
   }
   if (lane == 0) out[warp] = s;
+}
+// dist_decoder_*: the per-row codes come from net->row_code
+int decoder_codes(const dist_net_t* net, MlpArgs* a) {
+  if (net->n_codes <= 1) return DIST_OK;
+  DIST_REQUIRE(net->row_code != nullptr, "net: n_codes = %d needs row_code", net->n_codes);
+  a->row_code = net->row_code; a->code_div = 1;
+  return DIST_OK;
 }
 }  // namespace
 
@@ -158,19 +170,21 @@ int dist_fold_latent(const dist_net_t* net, const float* latent, float* out0, fl
   DIST_REQUIRE(net && out0, "fold_latent: null argument");
   cudaStream_t st = (cudaStream_t)stream;
   const int Lz = net->latent_size;
+  DIST_REQUIRE(net->n_codes >= 0 && net->n_codes <= 65535, "fold_latent: n_codes %d outside [0, 65535]", net->n_codes);
+  const unsigned C = net->n_codes > 1 ? (unsigned)net->n_codes : 1u;      // one grid row per code
   {
     const int N = net->N[0], Np = round_up(N, 4);
     if (Lz > 0) {
       DIST_REQUIRE(latent && net->Wz0 && net->b0, "fold_latent: null latent buffers");
-      k_fold<<<(Np * 32 + 255) / 256, 256, 0, st>>>(net->Wz0, net->b0, latent, N, Lz, out0, Np); count_launch();
+      k_fold<<<dim3((Np * 32 + 255) / 256, C), 256, 0, st>>>(net->Wz0, net->b0, latent, N, Lz, out0, Np); count_launch();
     } else {
-      k_fold<<<(Np * 32 + 255) / 256, 256, 0, st>>>(net->b0, net->b0, net->b0, N, 0, out0, Np); count_launch();
+      k_fold<<<dim3((Np * 32 + 255) / 256, C), 256, 0, st>>>(net->b0, net->b0, net->b0, N, 0, out0, Np); count_launch();
     }
   }
   if (net->latent_in >= 0 && Lz > 0) {
     DIST_REQUIRE(outl && net->Wzl && net->bl, "fold_latent: null latent_in buffers");
     const int N = net->N[net->latent_in], Np = round_up(N, 4);
-    k_fold<<<(Np * 32 + 255) / 256, 256, 0, st>>>(net->Wzl, net->bl, latent, N, Lz, outl, Np); count_launch();
+    k_fold<<<dim3((Np * 32 + 255) / 256, C), 256, 0, st>>>(net->Wzl, net->bl, latent, N, Lz, outl, Np); count_launch();
   }
   DIST_CHECK_CUDA(cudaGetLastError());
   return DIST_OK;
@@ -183,6 +197,8 @@ int dist_decoder_forward(const dist_net_t* net, int engine, const float* points,
   if (rc) return rc;
   MlpArgs a{};
   a.points = points; a.n_host = n_host; a.n_dev = n_dev; a.clamp_dist = clamp_dist; a.sdf = sdf;
+  rc = decoder_codes(net, &a);
+  if (rc) return rc;
   return mlp_launch(net, nd, engine, 0, a, (cudaStream_t)stream);
 }
 
@@ -196,6 +212,8 @@ int dist_decoder_forward_tiers(const dist_net_t* net, const float* points, int64
   MlpArgs a{};
   a.points = points; a.n_host = n_screen; a.n2_host = n_exact; a.seg2_offset = exact_offset; a.clamp_dist = 0.f; a.sdf = sdf;
   a.screen_seg1 = 1; a.screen_thresh = screen_thresh; a.seg_approx = seg_approx; a.tile_counters = tile_counters;
+  rc = decoder_codes(net, &a);
+  if (rc) return rc;
   return mlp_launch(net, nd, DIST_ENGINE_TC, 0, a, (cudaStream_t)stream);
 }
 
@@ -208,6 +226,8 @@ int dist_decoder_forward_masks(const dist_net_t* net, const float* points, int64
   MlpArgs a{};
   a.points = points; a.n_host = n; a.clamp_dist = 0.f; a.sdf = sdf;
   a.mask_buf = mask_buf; a.mask_cap = mask_cap; a.mask_base_host = mask_base;
+  rc = decoder_codes(net, &a);
+  if (rc) return rc;
   return mlp_launch(net, nd, DIST_ENGINE_TC, 0, a, (cudaStream_t)stream);
 }
 
@@ -220,6 +240,8 @@ int dist_decoder_backward_masked(const dist_net_t* net, const int32_t* slots, co
   MlpArgs a{};
   a.n_host = n; a.clamp_dist = clamp_dist; a.grad = dpoints; a.coef = coef; a.acc0 = acc0; a.accl = accl;
   a.mask_buf = const_cast<uint32_t*>(mask_buf); a.mask_cap = mask_cap; a.slots = slots; a.sdf_in = sdf_in;
+  rc = decoder_codes(net, &a);
+  if (rc) return rc;
   return mlp_launch(net, nd, DIST_ENGINE_TC, 3, a, (cudaStream_t)stream);
 }
 
@@ -230,6 +252,8 @@ int dist_decoder_input_grad(const dist_net_t* net, int engine, const float* poin
   if (rc) return rc;
   MlpArgs a{};
   a.points = points; a.n_host = n_host; a.n_dev = n_dev; a.clamp_dist = clamp_dist; a.sdf = sdf; a.grad = grad;
+  rc = decoder_codes(net, &a);
+  if (rc) return rc;
   return mlp_launch(net, nd, engine, 1, a, (cudaStream_t)stream);
 }
 
@@ -242,6 +266,8 @@ int dist_decoder_backward(const dist_net_t* net, int engine, const float* points
   MlpArgs a{};
   a.points = points; a.n_host = n_host; a.n_dev = n_dev; a.clamp_dist = clamp_dist; a.grad = dpoints;
   a.coef = coef; a.use_clamp = use_clamp; a.acc0 = acc0; a.accl = accl;
+  rc = decoder_codes(net, &a);
+  if (rc) return rc;
   return mlp_launch(net, nd, engine, 2, a, (cudaStream_t)stream);
 }
 

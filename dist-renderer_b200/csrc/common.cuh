@@ -36,6 +36,7 @@ struct NetDev {
   const float* Wt[DIST_MAX_LAYERS];
   const float* W[DIST_MAX_LAYERS];
   const float* bias[DIST_MAX_LAYERS];
+  int n_codes;   // > 1: bias[0] / bias[latent_in] are per-code tables [n_codes][Np4] (dist_net_t.n_codes)
 };
 
 int make_netdev(const dist_net_t* net, NetDev* out);
@@ -72,6 +73,11 @@ struct MlpArgs {
   const int32_t* mask_base_dev;
   const int32_t* slots;     // mode 3: [n] mask slot per row (-1: row contributes nothing)
   const float* sdf_in;      // mode 3: [n] recorded decoder output per row
+  // several latent codes (NetDev.n_codes > 1): row r uses code row_code[r] / code_div.  The launch sites pass an array they
+  // already have, aligned with the rows (an active list of pixels, pixel * DIST_MAX_BUFFER + record, ...), and the divisor
+  // that maps its entries to the view; accumulators acc0 / accl are then [n_codes][N].  Unused with one code.
+  const int32_t* row_code;
+  int32_t code_div;
 };
 int mlp_simt_launch(const NetDev& net, int mode, const MlpArgs& a, cudaStream_t stream);
 int mlp_tc_launch(const dist_net_t* net, const NetDev& nd, int mode, const MlpArgs& a, cudaStream_t stream);

@@ -355,15 +355,23 @@ __global__ void k_pyr_step(Cam cam, dist_march_t mp, Level L, int step, float* p
   }
 }
 
-// the origin (filler samples, renderer.py:539-540) is the only row of segment 2 at step 0: always at full precision
-__global__ void k_append_origin(dist_workspace_t ws, int SEG, int mask_slots_used) {
-  ws.pts[(size_t)SEG * 3] = 0.f; ws.pts[(size_t)SEG * 3 + 1] = 0.f; ws.pts[(size_t)SEG * 3 + 2] = 0.f;
-  ws.counts[1] = 1;
-  if (ws.mask_base) ws.mask_base[0] = mask_slots_used;    // the coarse pyramid levels recorded their rows before the march
+// the origin (filler samples, renderer.py:539-540) is the only row of segment 2 at step 0: always at full precision.
+// With one latent code per view there is one origin row per view (n_origin = n_views), listed as pixel v * Pv so that the
+// row's code is its view like every other row of the march.
+__global__ void k_append_origin(dist_workspace_t ws, int SEG, int mask_slots_used, int n_origin, int Pv) {
+  for (int o = threadIdx.x; o < n_origin; o += blockDim.x) {
+    const size_t r = (size_t)SEG + o;
+    ws.pts[r * 3] = 0.f; ws.pts[r * 3 + 1] = 0.f; ws.pts[r * 3 + 2] = 0.f;
+    ws.list_a[r] = o * Pv;
+  }
+  if (threadIdx.x == 0) {
+    ws.counts[1] = n_origin;
+    if (ws.mask_base) ws.mask_base[0] = mask_slots_used;    // the coarse pyramid levels recorded their rows before the march
+  }
 }
 
 // ---------------------------------------------------------------------------------------------- one march step
-__global__ void k_march_update(Cam cam, dist_march_t mp, dist_workspace_t ws, int step, int P) {
+__global__ void k_march_update(Cam cam, dist_march_t mp, dist_workspace_t ws, int step, int P, int n_origin) {
   const int SEG = seg_capacity(P);
   const int n1 = ws.counts[2 * step];
   const int n2 = (step == 0) ? 0 : ws.counts[2 * step + 1];      // (step 0: segment 2 holds the origin query only)
@@ -373,7 +381,8 @@ __global__ void k_march_update(Cam cam, dist_march_t mp, dist_workspace_t ws, in
   int32_t* nxt = (step & 1) ? ws.list_a : ws.list_b;
   const float* pts_cur = ws.pts + (size_t)(step & 1) * (size_t)(2 * SEG) * 3;       // points of this step
   float* pts_nxt = ws.pts + (size_t)((step + 1) & 1) * (size_t)(2 * SEG) * 3;       // points of the next step
-  if (step == 0 && blockIdx.x == 0 && threadIdx.x == 0) ws.sdf_origin[0] = ws.sdf[SEG];
+  if (step == 0 && blockIdx.x == 0)
+    for (int o = threadIdx.x; o < n_origin; o += blockDim.x) ws.sdf_origin[o] = ws.sdf[SEG + o];   // (one per view: per-view codes)
   // mask cache: the decoder launch of this step recorded the rows of segment 2 at slots mask_base[step] + (i - SEG)
   const bool mc = scr && ws.mask_buf != nullptr;
   const int mbase = mc ? ws.mask_base[step] : 0;
@@ -480,14 +489,15 @@ __global__ void k_requery_apply(dist_workspace_t ws, int P, int base_index) {
 }
 
 // ---------------------------------------------------------------------------------------------- finalize
-__global__ void k_finalize(dist_march_t mp, dist_workspace_t ws, float* Zdepth, uint8_t* mask, float* min_sdf, int P, int Pv) {
+__global__ void k_finalize(dist_march_t mp, dist_workspace_t ws, float* Zdepth, uint8_t* mask, float* min_sdf, int P, int Pv,
+                           int origin_per_view) {
   const int lp = blockIdx.x * blockDim.x + threadIdx.x;
   if (lp >= P || !(ws.flags[lp] & 1)) return;
   const int B = mp.buffer_size;
   // steps this ray's view executed before all of its rays had finished (the early break of renderer.py:562 is per render)
   const int S = ws.view_stat[VS_STRIDE * (lp / Pv) + VS_STEPS];
   int nreal = ws.nreal[lp];
-  const float so = ws.sdf_origin[0];
+  const float so = ws.sdf_origin[origin_per_view ? lp / Pv : 0];
   const float zfin = ws.z[lp];
   // renderer.py:562-567: an early break of the (full-resolution) march before buffer_size steps pads its lists with
   // copies of the last executed step; in the pyramid variant the padded fine-level lists are then concatenated with the
@@ -649,11 +659,11 @@ __global__ void k_normal_finish(Cam cam, const int32_t* idx_in, const float* gra
 // its ReLU masks in the mask cache (ws.top_slot >= 0) go to the "masked" list (ws.bm_*: transposed chain only), the others
 // (fillers, coarse pyramid samples, rows of re-evaluated tiles, everything when the cache is off) to the full replay list.
 __global__ void k_bwd_gen(dist_march_t mp, dist_workspace_t ws, const float* gZ, const float* gM, int32_t* row_pix,
-                          float* pts, float* coef, int32_t* count, int P, int use_masks) {
+                          float* pts, float* coef, int32_t* count, int P, int use_masks, int Pv, int origin_per_view) {
   const int lp = blockIdx.x * blockDim.x + threadIdx.x;
   const bool hit = lp < P && (ws.flags[lp] & 1);
   const int B = mp.buffer_size;
-  const float so = ws.sdf_origin[0];
+  const float so = hit ? ws.sdf_origin[origin_per_view ? lp / Pv : 0] : 0.f;
   const float gz = (hit && gZ) ? gZ[lp] : 0.f;
   const float gm = (hit && gM) ? gM[lp] : 0.f;
   for (int b = 0; b < B; ++b) {
@@ -749,6 +759,17 @@ int make_cam(const dist_camera_t* cam, Cam* out) {
   return DIST_OK;
 }
 
+// one latent code per view (dist_net_t.n_codes > 1): the code of a decoder row is the view of its pixel
+int check_codes(const NetDev& nd, const Cam& cam) {
+  DIST_REQUIRE(nd.n_codes <= 1 || nd.n_codes == cam.n_views, "net: n_codes = %d, but the call renders %d views", nd.n_codes,
+               cam.n_views);
+  return DIST_OK;
+}
+// rows whose array entries are pixels (active lists, normal rows) or pixel * DIST_MAX_BUFFER + record (re-query, backward rows)
+void set_codes(const NetDev& nd, MlpArgs& a, const int32_t* rows, int div) {
+  if (nd.n_codes > 1) { a.row_code = rows; a.code_div = div; }
+}
+
 }  // namespace
 
 // =============================================================================================== host entry points
@@ -789,12 +810,18 @@ int render_depth_fwd(const dist_net_t* net, int engine, const dist_camera_t* cam
   NetDev nd;
   rc = make_netdev(net, &nd);
   if (rc) return rc;
+  rc = check_codes(nd, cam);
+  if (rc) return rc;
+  const bool codes = nd.n_codes > 1;
   dist_march_t mpv = *mp_in;
   dist_march_t* mp = &mpv;
   DIST_REQUIRE(mp->buffer_size >= 1 && mp->buffer_size <= DIST_MAX_BUFFER, "buffer_size must be in [1,%d]", DIST_MAX_BUFFER);
   DIST_REQUIRE(mp->march_step >= 1, "march_step must be >= 1");
   DIST_REQUIRE(mp->marching_type >= DIST_MARCH_TRIVIAL && mp->marching_type <= DIST_MARCH_PYRAMID, "bad marching_type");
   DIST_REQUIRE(ws->entry0 && ws->top_lvl && ws->view_stat, "workspace: entry0 / top_lvl / view_stat missing");
+  DIST_REQUIRE(ws->ray && ws->entry && ws->exit_ && ws->dist && ws->z && ws->flags && ws->nreal && ws->top_sdf && ws->top_pt &&
+                   ws->top_zafter && ws->top_zgen && ws->list_a && ws->list_b && ws->pts && ws->sdf && ws->counts && ws->sdf_origin,
+               "workspace: a march buffer is missing");
   const bool pyr = mp->marching_type == DIST_MARCH_PYRAMID;
   const int P = cam.Pv * cam.n_views;
   DIST_CHECK_CUDA(cudaMemsetAsync(ws->view_stat, 0, sizeof(int32_t) * VS_STRIDE * cam.n_views, st));
@@ -855,6 +882,7 @@ int render_depth_fwd(const dist_net_t* net, int engine, const dist_camera_t* cam
         // mask cache: a coarse step's rows take L.P slots (its capacity), handed out in launch order
         const int64_t slot_base = mc ? coarse_slots : -1;
         if (mc) { a.mask_buf = ws->mask_buf; a.mask_cap = ws->mask_cap; a.mask_base_host = slot_base; coarse_slots += (L.P + 127) / 128 * 128; }
+        set_codes(nd, a, L.list, L.Pv);
         rc = mlp_launch(net, nd, engine, 0, a, st);
         if (rc) return rc;
         k_pyr_step<<<min((L.P + tb - 1) / tb, 4 * num_sms()), tb, 0, st>>>(cam, *mp, L, s, ws->pts, ws->sdf, slot_base,
@@ -866,7 +894,8 @@ int render_depth_fwd(const dist_net_t* net, int engine, const dist_camera_t* cam
   DIST_CHECK_CUDA(cudaMemsetAsync(ws->counts, 0, sizeof(int32_t) * 2 * (S_total + 2), st));
   k_setup<<<(cam.n_views * setup_threads_per_view(cam.W, cam.n_rows) + tb - 1) / tb, tb, 0, st>>>(cam, *mp, *ws, Zdepth, mask, min_sdf, P,
                                                                                                 L1, L2); count_launch();
-  k_append_origin<<<1, 1, 0, st>>>(*ws, SEG, (int)coarse_slots); count_launch();
+  const int n_origin = codes ? cam.n_views : 1;
+  k_append_origin<<<1, 256, 0, st>>>(*ws, SEG, (int)coarse_slots, n_origin, cam.Pv); count_launch();
   DIST_CHECK_CUDA(cudaGetLastError());
   const int gu = min(gb, 4 * num_sms());
   for (int s = 0; s < S; ++s) {
@@ -879,9 +908,10 @@ int render_depth_fwd(const dist_net_t* net, int engine, const dist_camera_t* cam
     a.tile_counters = ws->tile_counters;
     if (scr) { a.screen_seg1 = 1; a.screen_thresh = mp->clamp_dist + mp->screen_margin; a.seg_approx = ws->seg_approx; }
     if (mc) { a.mask_buf = ws->mask_buf; a.mask_cap = ws->mask_cap; a.mask_base_dev = ws->mask_base + s; }
+    set_codes(nd, a, (s & 1) ? ws->list_b : ws->list_a, cam.Pv);     // both segments: the rows' entries of the active list
     rc = mlp_launch(net, nd, engine, 0, a, st);
     if (rc) return rc;
-    k_march_update<<<gu, tb, 0, st>>>(cam, *mp, *ws, s, P); count_launch();
+    k_march_update<<<gu, tb, 0, st>>>(cam, *mp, *ws, s, P, n_origin); count_launch();
   }
   if (scr) {
     k_requery_gen<<<gb, tb, 0, st>>>(*mp, *ws, P); count_launch();
@@ -889,11 +919,12 @@ int render_depth_fwd(const dist_net_t* net, int engine, const dist_camera_t* cam
     a.points = ws->rq_pts; a.n_host = (int64_t)P * mp->buffer_size; a.n_dev = ws->rq_cnt; a.clamp_dist = 0.f; a.sdf = ws->rq_sdf;
     a.tile_counters = ws->tile_counters;
     if (mc) { a.mask_buf = ws->mask_buf; a.mask_cap = ws->mask_cap; a.mask_base_dev = ws->mask_base + S; }   // after the last step's rows
+    set_codes(nd, a, ws->rq_idx, cam.Pv * DIST_MAX_BUFFER);
     rc = mlp_launch(net, nd, engine, 0, a, st);
     if (rc) return rc;
     k_requery_apply<<<gu, tb, 0, st>>>(*ws, P, S); count_launch();
   }
-  k_finalize<<<gb, tb, 0, st>>>(*mp, *ws, Zdepth, mask, min_sdf, P, cam.Pv); count_launch();
+  k_finalize<<<gb, tb, 0, st>>>(*mp, *ws, Zdepth, mask, min_sdf, P, cam.Pv, codes ? 1 : 0); count_launch();
   DIST_CHECK_CUDA(cudaGetLastError());
   return DIST_OK;
 }
@@ -907,6 +938,8 @@ int render_normal_fwd(const dist_net_t* net, int engine, const dist_camera_t* ca
   NetDev nd;
   rc = make_netdev(net, &nd);
   if (rc) return rc;
+  rc = check_codes(nd, cam);
+  if (rc) return rc;
   const int P = cam.Pv * cam.n_views;
   DIST_CHECK_CUDA(cudaMemsetAsync(s_count, 0, sizeof(int32_t), st));
   DIST_CHECK_CUDA(cudaMemsetAsync(Znormal, 0, sizeof(float) * 3 * (size_t)P, st));
@@ -915,6 +948,7 @@ int render_normal_fwd(const dist_net_t* net, int engine, const dist_camera_t* ca
   MlpArgs a{};
   a.points = s_pts; a.n_host = P; a.n_dev = s_count; a.clamp_dist = clamp_dist; a.grad = s_grad;
   a.rows_evaluated = rows_eval;
+  set_codes(nd, a, s_idx, cam.Pv);
   rc = mlp_launch(net, nd, engine, 1, a, st);
   if (rc) return rc;
   k_normal_finish<<<min(gb, 4 * num_sms()), tb, 0, st>>>(cam, s_idx, s_grad, s_count, normalize, Znormal, P); count_launch();
@@ -933,6 +967,9 @@ int render_depth_bwd(const dist_net_t* net, int engine, const dist_camera_t* cam
   NetDev nd;
   rc = make_netdev(net, &nd);
   if (rc) return rc;
+  rc = check_codes(nd, cam);
+  if (rc) return rc;
+  const bool codes = nd.n_codes > 1;
   const int P = cam.Pv * cam.n_views;
   DIST_CHECK_CUDA(cudaMemsetAsync(s_count, 0, sizeof(int32_t), st));
   const int tb = 256, gb = (P + tb - 1) / tb;
@@ -940,10 +977,12 @@ int render_depth_bwd(const dist_net_t* net, int engine, const dist_camera_t* cam
   const bool mc = engine == DIST_ENGINE_TC && ws->mask_buf && ws->top_slot && ws->bm_row && ws->bm_slot && ws->bm_sdf && ws->bm_coef &&
                   ws->bm_dpts && ws->bm_cnt;
   if (mc) DIST_CHECK_CUDA(cudaMemsetAsync(ws->bm_cnt, 0, sizeof(int32_t), st));
-  k_bwd_gen<<<gb, tb, 0, st>>>(*mp, *ws, gZ, gM, s_row_pix, s_pts, s_coef, s_count, P, mc ? 1 : 0); count_launch();
+  k_bwd_gen<<<gb, tb, 0, st>>>(*mp, *ws, gZ, gM, s_row_pix, s_pts, s_coef, s_count, P, mc ? 1 : 0, cam.Pv,
+                                codes ? 1 : 0); count_launch();
   MlpArgs a{};
   a.points = s_pts; a.n_host = (int64_t)P * mp->buffer_size; a.n_dev = s_count; a.clamp_dist = 0.f;
   a.grad = s_dpts; a.coef = s_coef; a.acc0 = acc0; a.accl = accl; a.rows_evaluated = rows_eval;
+  set_codes(nd, a, s_row_pix, cam.Pv * DIST_MAX_BUFFER);
   rc = mlp_launch(net, nd, engine, 2, a, st);
   if (rc) return rc;
   if (mc) {
@@ -952,6 +991,7 @@ int render_depth_bwd(const dist_net_t* net, int engine, const dist_camera_t* cam
     b.grad = ws->bm_dpts; b.coef = ws->bm_coef; b.acc0 = acc0; b.accl = accl;
     b.rows_evaluated = rows_eval ? rows_eval + 1 : nullptr;      // counted apart: these rows cost F, not 2F
     b.mask_buf = ws->mask_buf; b.mask_cap = ws->mask_cap; b.slots = ws->bm_slot; b.sdf_in = ws->bm_sdf;
+    set_codes(nd, b, ws->bm_row, cam.Pv * DIST_MAX_BUFFER);
     rc = mlp_launch(net, nd, engine, 3, b, st);
     if (rc) return rc;
   }

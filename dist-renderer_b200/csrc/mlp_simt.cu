@@ -33,6 +33,7 @@ struct Smem {
 };
 constexpr size_t kSmemFwd = sizeof(Smem);
 constexpr size_t kSmemGrad = sizeof(Smem) + size_t(MAXH_GRAD) * TM * 64;
+constexpr size_t kSmemCodes = TM * sizeof(int);   // several latent codes: the tile's row codes, behind everything else
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   unsigned s = (unsigned)__cvta_generic_to_shared(smem);
@@ -123,11 +124,14 @@ __device__ __forceinline__ void zero_rows(Smem& sm, int k_begin, int k_end, int 
   for (int i = k_begin * TM + tid; i < k_end * TM; i += NT) sm.act[i] = 0.f;
 }
 
-template <int MODE>  // 0 forward, 1 input gradient, 2 backward replay (adds coef / accumulators)
+// MODE: 0 forward, 1 input gradient, 2 backward replay (adds coef / accumulators).
+// MC: several latent codes (net.n_codes > 1): per-row folded biases of layer 0 and the latent_in layer, per-code row sums.
+template <int MODE, bool MC>
 __global__ void __launch_bounds__(NT, 1) mlp_simt_kernel(NetDev net, MlpArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
   unsigned char* masks = smem_raw + sizeof(Smem);  // [layer][row][64] (gradient modes)
+  int* codes = reinterpret_cast<int*>(smem_raw + (MODE == 0 ? kSmemFwd : kSmemGrad));   // [TM] (MC)
   const int tid = threadIdx.x;
   const int rg = tid >> 6;
   const int64_t n = a.n_dev ? (int64_t)*a.n_dev : a.n_host;
@@ -150,6 +154,8 @@ __global__ void __launch_bounds__(NT, 1) mlp_simt_kernel(NetDev net, MlpArgs a) 
       sm.dxyz[tid] = 0.f;
       sm.act[(tid % 3) * TM + r] = v;
     }
+    // rows past the end take the last row's code: their contributions are zero, and they do not split a run of codes
+    if (MC && tid < TM) codes[tid] = a.row_code[row0 + min(tid, nvalid - 1)] / a.code_div;
     zero_rows(sm, 3, 8, tid);
     __syncthreads();
 
@@ -158,6 +164,7 @@ __global__ void __launch_bounds__(NT, 1) mlp_simt_kernel(NetDev net, MlpArgs a) 
       const int N = net.N[l], Np4 = round_up(N, 4);
       gemm_tile(sm, net.Wt[l], round_up(net.K[l], 8), Np4, acc, tid);
       const float* bias = net.bias[l];
+      const bool per_code = MC && (l == 0 || l == net.latent_in);     // folded bias: [n_codes][Np4]
       unsigned mbits[16];
 #pragma unroll
       for (int r = 0; r < 16; ++r) mbits[r] = 0u;
@@ -167,7 +174,9 @@ __global__ void __launch_bounds__(NT, 1) mlp_simt_kernel(NetDev net, MlpArgs a) 
         const float b = (col < Np4) ? __ldg(bias + col) : 0.f;
 #pragma unroll
         for (int r = 0; r < 16; ++r) {
-          float v = acc[r][c] + b;
+          float bb = b;
+          if (per_code) bb = (col < Np4) ? __ldg(bias + (size_t)codes[rg * 16 + r] * Np4 + col) : 0.f;
+          float v = acc[r][c] + bb;
           if (v > 0.f) mbits[r] |= (1u << c); else v = 0.f;
           acc[r][c] = v;
         }
@@ -245,7 +254,24 @@ __global__ void __launch_bounds__(NT, 1) mlp_simt_kernel(NetDev net, MlpArgs a) 
       // act holds delta_pre[l] as [n][row], n < N[l].  Accumulate its row-sum for the latent gradient.
       if (MODE == 2) {
         float* accp = (l == 0) ? a.acc0 : ((l == net.latent_in) ? a.accl : nullptr);
-        if (accp) {
+        if (accp && MC) {
+          // per-code row sums: runs of equal codes, flushed to accp[code][nn] when the code changes (rotated start as below)
+          const int Nl = net.N[l];
+          for (int nn = tid; nn < Nl; nn += NT) {
+            int cur = codes[tid & (TM - 1)];
+            float s = 0.f;
+            for (int k = 0; k < TM; ++k) {
+              const int r = (k + tid) & (TM - 1);
+              const int cr = codes[r];
+              if (cr != cur) {
+                if (s != 0.f) atomicAdd(accp + (size_t)cur * Nl + nn, s);
+                s = 0.f; cur = cr;
+              }
+              s += sm.act[(size_t)nn * TM + r];
+            }
+            if (s != 0.f) atomicAdd(accp + (size_t)cur * Nl + nn, s);
+          }
+        } else if (accp) {
           for (int nn = tid; nn < net.N[l]; nn += NT) {
             float s = 0.f;
 #pragma unroll 8
@@ -294,22 +320,33 @@ int mlp_simt_launch(const NetDev& net, int mode, const MlpArgs& a, cudaStream_t 
   DIST_REQUIRE(net.n_layers >= 2 && net.n_layers <= DIST_MAX_LAYERS, "mlp_simt: n_layers %d unsupported", net.n_layers);
   if (mode != 0) DIST_REQUIRE(net.n_layers - 1 <= MAXH_GRAD, "mlp_simt: at most %d hidden layers in gradient modes", MAXH_GRAD);
   if (a.n_host <= 0 && !a.n_dev) return DIST_OK;
+  const bool mc = net.n_codes > 1;
+  if (mc) DIST_REQUIRE(a.row_code && a.code_div > 0, "mlp_simt: %d latent codes need per-row codes", net.n_codes);
   static bool attr_done_dev[64] = {false};
   int cur_dev = 0;
   cudaGetDevice(&cur_dev);
   bool& attr_done = attr_done_dev[cur_dev & 63];
   if (!attr_done) {
-    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemFwd));
-    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemGrad));
-    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemGrad));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemFwd));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemGrad));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemGrad));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kSmemFwd + kSmemCodes)));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kSmemGrad + kSmemCodes)));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_simt_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kSmemGrad + kSmemCodes)));
     attr_done = true;
   }
   int64_t tiles = (a.n_host + TM - 1) / TM;
   int grid = (int)((tiles < (int64_t)num_sms()) ? tiles : (int64_t)num_sms());
   if (grid < 1) grid = 1;
-  if (mode == 0) { mlp_simt_kernel<0><<<grid, NT, kSmemFwd, stream>>>(net, a); }
-  else if (mode == 1) { mlp_simt_kernel<1><<<grid, NT, kSmemGrad, stream>>>(net, a); }
-  else { mlp_simt_kernel<2><<<grid, NT, kSmemGrad, stream>>>(net, a); }
+  if (!mc) {
+    if (mode == 0) { mlp_simt_kernel<0, false><<<grid, NT, kSmemFwd, stream>>>(net, a); }
+    else if (mode == 1) { mlp_simt_kernel<1, false><<<grid, NT, kSmemGrad, stream>>>(net, a); }
+    else { mlp_simt_kernel<2, false><<<grid, NT, kSmemGrad, stream>>>(net, a); }
+  } else {
+    if (mode == 0) { mlp_simt_kernel<0, true><<<grid, NT, kSmemFwd + kSmemCodes, stream>>>(net, a); }
+    else if (mode == 1) { mlp_simt_kernel<1, true><<<grid, NT, kSmemGrad + kSmemCodes, stream>>>(net, a); }
+    else { mlp_simt_kernel<2, true><<<grid, NT, kSmemGrad + kSmemCodes, stream>>>(net, a); }
+  }
   count_launch();
   DIST_CHECK_CUDA(cudaGetLastError());
   return DIST_OK;

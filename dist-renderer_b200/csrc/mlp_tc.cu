@@ -95,6 +95,9 @@ struct TcParams {
   int first_append;                // layer 0's output gets xyz appended (latent_in == 1)
   int dbg;                         // diagnostics (DIST_TC_DEBUG), see the file header
   int stage_rows;                  // tensor-map rows per 16 KB weight stage (STAGE_BYTES / bytes per box row)
+  // several latent codes (MC instantiations): bias0 is [n_codes][N0p4]; the forward program layer lat_m (the latent_in
+  // layer, -1: none) reads its bias from [n_codes][lat_stride]
+  int lat_m, lat_stride;
 };
 
 struct TcIO {
@@ -116,6 +119,8 @@ struct TcIO {
   const int32_t* mask_base_dev;
   const int32_t* slots;         // MODE 3: [n] mask slot of each row
   const float* sdf_in;          // MODE 3: [n] the (unclamped) decoder output of each row, as recorded by the forward
+  const int32_t* row_code;      // MC: code of row r = row_code[r] / code_div (MlpArgs.row_code)
+  int32_t code_div;
 };
 
 // --------------------------------------------------------------------------------------------- PTX helpers
@@ -225,7 +230,11 @@ __device__ __forceinline__ void store_group_hi(uint8_t* smem, int region, int fe
 // upstream coefficients: d/dxyz per row and the row-summed pre-activation gradients of layer 0 / the latent_in layer.
 // MODE 3: MODE 2 without its forward half: the ReLU sign bits come from the mask cache a MODE 0 launch wrote (io.slots), the
 // decoder output from io.sdf_in; only the transposed chain runs (program layers n_mma .. 2 n_mma - 1).
-template <int MODE>
+// MC: several latent codes (dist_net_t.n_codes > 1).  Each thread owns one row in the epilogue, so it reads the folded
+// biases (layer 0, the latent_in layer) at its row's code -- rows of a warp mostly share a code and the loads broadcast --
+// and MODE 2/3 accumulate the latent gradient per code (see "per-code running sums").  MC = false is the one-code kernel
+// with none of this in it.
+template <int MODE, bool MC>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
 mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_hi, const TcParams P, const TcIO io) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -542,6 +551,20 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
     float px = 0.f, py = 0.f, pz = 0.f;
     uint32_t mk[DIST_MAX_LAYERS][2];     // ReLU sign bits of this thread's (row, 32 features x 2 halves) per net layer
     float acc0r[2] = {0.f, 0.f}, acclr[2] = {0.f, 0.f};  // MODE 2: per-lane running column sums
+    // per-code running sums (MC): the sums above belong to code acc_code (warp-uniform) and are flushed into acc[acc_code]
+    // when a tile whose 32 rows of this warp share another code comes along; tiles with mixed rows bypass them
+    int acc_code = 0;
+    auto flush_sums = [&]() {
+      // lane j of this warp holds column 32*kb + j of its blocks
+      const size_t o0 = MC ? (size_t)acc_code * P.N0 : 0, ol = MC ? (size_t)acc_code * P.accl_N : 0;
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int f = 32 * (8 * h + 4 * q + ch) + lane;
+        if (io.acc0 && f < P.N0 && acc0r[h] != 0.f) atomicAdd(io.acc0 + o0 + f, acc0r[h] * (1.f / sD));
+        if (io.accl && P.acc_l_prog >= 0 && f < P.accl_N && acclr[h] != 0.f) atomicAdd(io.accl + ol + f, acclr[h] * (1.f / sD));
+        acc0r[h] = 0.f; acclr[h] = 0.f;
+      }
+    };
 
     // mask-cache slot of this thread's row in tile t (-1: not recorded): only rows evaluated at full precision in the first
     // sweep -- the second row segment when the first is screened, every row of a plain single-segment launch
@@ -556,10 +579,22 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
       return (sl < io.mask_cap) ? sl : -1;
     };
     const bool rec_on = (MODE == 0) && mask_base >= 0;
+    // MC: code of this thread's row in tile t; a row past the end takes the last row's code (its contributions are zero,
+    // and it does not split the warp's code group)
+    auto code_of = [&](int64_t t) -> int {
+      if constexpr (!MC) { return 0; }
+      else {
+        const int64_t lim = lim_of(t);
+        const int64_t r = min(row0_of(t) + rank * 64 + row, lim - 1);
+        return io.row_code[r] / io.code_div;
+      }
+    };
+    int pc = 0, qc = 0;                  // MC: codes of the rows whose points are in (px, py, pz) / (qx, qy, qz)
     auto load_point = [&](int64_t t) {
       const int64_t gr = row0_of(t) + rank * 64 + row;
       if (gr < lim_of(t)) { px = io.points[gr * 3]; py = io.points[gr * 3 + 1]; pz = io.points[gr * 3 + 2]; }
       else { px = py = pz = 0.f; }
+      if (MC) pc = code_of(t);
     };
     auto signal_block = [&](int kc) {   // this warp's 32 rows x 32 features of A block kc are written
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -579,6 +614,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
         const int f0 = 32 * kb;
         uint32_t m0 = 0;
         if (kb < guard_kc32) mbar_wait(A_FREE(kb), (free_phase >> kb) & 1);
+        const float* bias0 = MC ? P.bias0 + (size_t)pc * P.N0p4 : P.bias0;
 #pragma unroll
         for (int g = 0; g < 4; ++g) {
           float x[8];
@@ -587,7 +623,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
             const int f = f0 + 8 * g + e;
             float v = 0.f;
             if (f < P.N0) {
-              v = fmaf(__ldg(P.w0 + 2 * P.N0p4 + f), pz, fmaf(__ldg(P.w0 + P.N0p4 + f), py, __ldg(P.w0 + f) * px)) + __ldg(P.bias0 + f);
+              v = fmaf(__ldg(P.w0 + 2 * P.N0p4 + f), pz, fmaf(__ldg(P.w0 + P.N0p4 + f), py, __ldg(P.w0 + f) * px)) + __ldg(bias0 + f);
               if (v > 0.f) m0 |= 1u << (8 * g + e); else v = 0.f;
             } else if (P.first_append && f < P.N0 + 3) {
               v = (f == P.N0) ? px : ((f == P.N0 + 1) ? py : pz);
@@ -630,6 +666,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
       const int64_t grb = row0_of(tb) + rank * 64 + row;
       if (i + 1 < c1 && grb < n1) { qx = io.points[grb * 3]; qy = io.points[grb * 3 + 1]; qz = io.points[grb * 3 + 2]; }
       else { qx = qy = qz = 0.f; }
+      if (MC) qc = (i + 1 < c1) ? code_of(tb) : pc;
     };
     auto layer0_pair = [&](int guard_kc32) {     // layer 0 of both tiles on CUDA cores: hi halves into the two activation regions
       const int kblocks = P.L[0].kc32;
@@ -647,9 +684,12 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
             const int f = f0 + 8 * g + e;
             float va = 0.f, vb = 0.f;
             if (f < P.N0) {
-              const float wx = __ldg(P.w0 + f), wy = __ldg(P.w0 + P.N0p4 + f), wz = __ldg(P.w0 + 2 * P.N0p4 + f), b = __ldg(P.bias0 + f);
+              const float wx = __ldg(P.w0 + f), wy = __ldg(P.w0 + P.N0p4 + f), wz = __ldg(P.w0 + 2 * P.N0p4 + f);
+              float b = 0.f, bq = 0.f;
+              if (MC) { b = __ldg(P.bias0 + (size_t)pc * P.N0p4 + f); bq = __ldg(P.bias0 + (size_t)qc * P.N0p4 + f); }
+              else { b = __ldg(P.bias0 + f); bq = b; }
               va = fmaxf(fmaf(wz, pz, fmaf(wy, py, wx * px)) + b, 0.f);
-              vb = fmaxf(fmaf(wz, qz, fmaf(wy, qy, wx * qx)) + b, 0.f);
+              vb = fmaxf(fmaf(wz, qz, fmaf(wy, qy, wx * qx)) + bq, 0.f);
             } else if (P.first_append && f < P.N0 + 3) {
               va = (f == P.N0) ? px : ((f == P.N0 + 1) ? py : pz);
               vb = (f == P.N0) ? qx : ((f == P.N0 + 1) ? qy : qz);
@@ -715,6 +755,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
       const int64_t ta = tile_of(i), tb = tile_of(i + 1);
       const int64_t gra = row0_of(ta) + rank * 64 + row, grb = row0_of(tb) + rank * 64 + row;
       const bool oka = gra < n1, okb = has_b && grb < n1;
+      const int ca = MC ? code_of(ta) : 0, cb = (MC && has_b) ? code_of(tb) : ca;   // for the latent_in layer's bias
       float dota = 0.f, dotb = 0.f;
       for (int m = 0; m < n_mma; ++m, ++G) {
         const bool last = (m == n_mma - 1);
@@ -744,10 +785,12 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
           for (int ts = 0; ts < (has_b ? 2 : 1); ++ts) {
             float v[32];
             tmem_ld32(tmem + lane_base + ts * 256 + h * 128 + 32 * ch, v);
+            const float* Lb = Lbias;
+            if (MC && m == P.lat_m) Lb += (size_t)(ts ? cb : ca) * P.lat_stride;
             if (interior) {
 #pragma unroll
               for (int j4 = 0; j4 < 8; ++j4) {
-                const float4 b4 = __ldg(reinterpret_cast<const float4*>(Lbias + fb) + j4);
+                const float4 b4 = __ldg(reinterpret_cast<const float4*>(Lb + fb) + j4);
                 v[4 * j4] = fmaxf(fmaf(v[4 * j4], cscale, b4.x), 0.f);
                 v[4 * j4 + 1] = fmaxf(fmaf(v[4 * j4 + 1], cscale, b4.y), 0.f);
                 v[4 * j4 + 2] = fmaxf(fmaf(v[4 * j4 + 2], cscale, b4.z), 0.f);
@@ -759,7 +802,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
               for (int j = 0; j < 32; ++j) {
                 const int f = fb + j;
                 float a = 0.f;
-                if (f < LN) a = fmaxf(fmaf(v[j], cscale, __ldg(Lbias + f)), 0.f);
+                if (f < LN) a = fmaxf(fmaf(v[j], cscale, __ldg(Lb + f)), 0.f);
                 else if (Lapp && f < LN + 3) a = ((f == LN) ? ax : ((f == LN + 1) ? ay : az)) * sA;
                 v[j] = a;
               }
@@ -829,6 +872,13 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
       const int64_t slot = rec_slot(t);
       float dot = 0.f, rowscale = (MODE == 3) ? seed_scale : 0.f, dx = 0.f, dy = 0.f, dz = 0.f;
       uint32_t mk0s[2] = {0u, 0u};
+      // MC: this row's code, and whether the warp's 32 rows share it (then the latent gradient goes to the running sums)
+      const int code_t = MC ? code_of(t) : 0;
+      bool code_uni = true;
+      if constexpr (MC && (MODE == 2 || MODE == 3)) {
+        code_uni = __match_any_sync(0xffffffffu, code_t) == 0xffffffffu;
+        if (code_uni && code_t != acc_code) { flush_sums(); acc_code = code_t; }
+      }
       for (int m = m0; m < n_prog; ++m, ++G) {
         const uint32_t buf = G & 1;
         const bool fwd = m < n_mma;
@@ -837,6 +887,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
         const int LN = P.L[m].N, Lnh = P.L[m].nh, Lapp = P.L[m].app_xyz;
         const float cscale = P.L[m].inv_scale;
         const float* Lbias = P.L[m].bias;
+        if (MC && m == P.lat_m) Lbias += (size_t)code_t * P.lat_stride;     // this row's folded bias of the latent_in layer
         const int kc32_cur = P.L[m].kc32;
         auto wait_half = [&](int h) {
           const int bi = 2 * buf + h;
@@ -985,8 +1036,26 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
               // row-sum of rowscale * delta for the latent gradient; column j of this 32-block ends in lane j
 #pragma unroll
               for (int j = 0; j < 32; ++j) v[j] *= rowscale;
-              const float sres = colsum32(v);
-              if (prog_last) acc0r[h] += sres; else acclr[h] += sres;
+              if (MC && !code_uni) {
+                // the warp's rows hold several codes: one reduction per code group, straight into acc[code]
+                float* accp = prog_last ? io.acc0 : io.accl;
+                const int Nacc = prog_last ? P.N0 : P.accl_N;
+                const int f = fb + lane;
+                unsigned rem = 0xffffffffu;
+                while (rem) {
+                  const int c = __shfl_sync(0xffffffffu, code_t, __ffs(rem) - 1);
+                  const bool mine = code_t == c;
+                  float w[32];
+#pragma unroll
+                  for (int j = 0; j < 32; ++j) w[j] = mine ? v[j] : 0.f;
+                  const float sres = colsum32(w);
+                  if (accp && f < Nacc && sres != 0.f) atomicAdd(accp + (size_t)c * Nacc + f, sres * (1.f / sD));
+                  rem &= ~__ballot_sync(0xffffffffu, mine);
+                }
+              } else {
+                const float sres = colsum32(v);
+                if (prog_last) acc0r[h] += sres; else acclr[h] += sres;
+              }
             }
           }
         }
@@ -1077,15 +1146,7 @@ mlp_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ 
       if (n_tiles_1pass) atomicAdd(io.tile_counters, (unsigned long long)n_tiles_1pass);
       if (n_tiles_3pass) atomicAdd(io.tile_counters + 1, (unsigned long long)n_tiles_3pass);
     }
-    if (MODE == 2 || MODE == 3) {
-      // flush the per-lane running column sums: lane j of this warp holds column 32*kb + j of its blocks
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const int f = 32 * (8 * h + 4 * q + ch) + lane;
-        if (io.acc0 && f < P.N0 && acc0r[h] != 0.f) atomicAdd(io.acc0 + f, acc0r[h] * (1.f / sD));
-        if (io.accl && P.acc_l_prog >= 0 && f < P.accl_N && acclr[h] != 0.f) atomicAdd(io.accl + f, acclr[h] * (1.f / sD));
-      }
-    }
+    if (MODE == 2 || MODE == 3) flush_sums();
   }
   if (io.dbg_out && blockIdx.x == 0 && tid == 0) {
     long long t1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
@@ -1164,6 +1225,10 @@ int mlp_tc_launch(const dist_net_t* net, const NetDev& nd, int mode, const MlpAr
   P.wlast = nd.W[nl - 1]; P.blast = nd.bias[nl - 1]; P.K_last = nd.K[nl - 1];
   P.use_tanh = nd.use_tanh; P.sA = 32.0f; P.sD = 256.0f;
   P.first_append = (nd.latent_in == 1) ? 1 : 0;
+  P.lat_m = (nd.latent_in >= 1) ? nd.latent_in - 1 : -1;
+  P.lat_stride = (nd.latent_in >= 1) ? round_up(nd.N[nd.latent_in], 4) : 0;
+  const bool mc = nd.n_codes > 1;
+  DIST_REQUIRE(!mc || (a.row_code && a.code_div > 0), "tensor-core engine: %d latent codes need per-row codes", nd.n_codes);
   { const char* e = getenv("DIST_TC_DEBUG"); P.dbg = e ? atoi(e) : 0; }
 
   TcIO io;
@@ -1176,6 +1241,7 @@ int mlp_tc_launch(const dist_net_t* net, const NetDev& nd, int mode, const MlpAr
   io.tile_counters = a.tile_counters;
   io.mask_buf = a.mask_buf; io.mask_cap = a.mask_cap; io.mask_base_host = a.mask_buf ? a.mask_base_host : -1;
   io.mask_base_dev = a.mask_base_dev; io.slots = a.slots; io.sdf_in = a.sdf_in;
+  io.row_code = mc ? a.row_code : nullptr; io.code_div = mc ? a.code_div : 1;
   DIST_REQUIRE(!io.screen_seg1 || io.seg_approx != nullptr, "tensor-core engine: two-tier precision needs seg_approx");
   DIST_REQUIRE((a.n2_host == 0 && !a.n2_dev) || (a.seg2_offset % 128 == 0 && a.seg2_offset >= a.n_host),
                "tensor-core engine: the second row segment must start at a multiple of 128 behind the first");
@@ -1212,20 +1278,32 @@ int mlp_tc_launch(const dist_net_t* net, const NetDev& nd, int mode, const MlpAr
   cudaGetDevice(&cur_dev);
   bool& attr_done = attr_done_dev[cur_dev & 63];
   if (!attr_done) {
-    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    DIST_CHECK_CUDA(cudaFuncSetAttribute(mlp_tc_kernel<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     attr_done = true;
   }
   const int64_t tiles = (a.n_host + 127) / 128 + (a.n2_host + 127) / 128;   // capacities when the counts live on the device
   int clusters = num_sms() / 2;
   if (tiles < clusters) clusters = (int)tiles;
   if (clusters < 1) clusters = 1;
-  if (mode == 0) { mlp_tc_kernel<0><<<clusters * 2, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
-  else if (mode == 1) { mlp_tc_kernel<1><<<clusters * 2, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
-  else if (mode == 2) { mlp_tc_kernel<2><<<clusters * 2, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
-  else { mlp_tc_kernel<3><<<clusters * 2, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+  const int g = clusters * 2;
+  if (!mc) {
+    if (mode == 0) { mlp_tc_kernel<0, false><<<g, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+    else if (mode == 1) { mlp_tc_kernel<1, false><<<g, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+    else if (mode == 2) { mlp_tc_kernel<2, false><<<g, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+    else { mlp_tc_kernel<3, false><<<g, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+  } else {
+    if (mode == 0) { mlp_tc_kernel<0, true><<<g, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+    else if (mode == 1) { mlp_tc_kernel<1, true><<<g, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+    else if (mode == 2) { mlp_tc_kernel<2, true><<<g, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+    else { mlp_tc_kernel<3, true><<<g, NTHREADS, SMEM_BYTES, stream>>>(tmap, tmap_hi, P, io); }
+  }
   count_launch();
   DIST_CHECK_CUDA(cudaGetLastError());
   if (P.dbg & 4) {

@@ -117,25 +117,31 @@ class DecoderPlan(object):
         self._key = key
         return True
 
-    def fold(self, latent, stream):
-        """Per-render folded biases (device tensors) for layer 0 and the latent_in layer."""
+    def fold(self, latent, stream, n_codes=1):
+        """Per-render folded biases (device tensors) for layer 0 and the latent_in layer.  With n_codes = C > 1, `latent`
+        holds C codes (C, L) and the biases are per-code tables, flat [C][Np4]: row c is byte for byte what folding code c
+        alone gives (one launch, the codes on the grid's second dimension)."""
         lib = _abi.lib()
-        out0 = torch.empty_like(self.bias[0])
-        outl = torch.empty_like(self.bias[self.latent_in]) if self.latent_in >= 0 else None
-        net = self.c_net(None, None)
+        C = max(1, int(n_codes))
+        f32 = dict(device=self.device, dtype=torch.float32)
+        out0 = torch.empty(C * self.bias[0].numel(), **f32)
+        outl = torch.empty(C * self.bias[self.latent_in].numel(), **f32) if self.latent_in >= 0 else None
+        net = self.c_net(None, None, n_codes=C)
         lat = None
         if self.latent_size > 0:
             if latent is None:
                 raise ValueError("this decoder expects a latent code")
             lat = latent.detach().reshape(-1).float().contiguous()
-            if lat.numel() != self.latent_size:
-                raise ValueError("latent has %d elements, decoder expects %d" % (lat.numel(), self.latent_size))
+            if lat.numel() != C * self.latent_size:
+                raise ValueError("latent has %d elements, decoder expects %d" % (lat.numel(), C * self.latent_size))
         _abi.check(lib.dist_fold_latent(net, _abi.ptr(lat), _abi.ptr(out0), _abi.ptr(outl), stream))
         return out0, outl, lat
 
-    def net_for(self, latent, engine, stream, out_index=0):
+    def net_for(self, latent, engine, stream, out_index=0, n_codes=1):
         """(dist_net_t, effective engine, keepalive) for one call: prepares the tensor-core operands when that engine is selected,
-        folds the latent into the per-render biases and fills the descriptor (for output `out_index` of the network)."""
+        folds the latent into the per-render biases and fills the descriptor (for output `out_index` of the network).
+        n_codes > 1: `latent` is (n_codes, L) and the descriptor carries per-code bias tables (dist_net_t.n_codes); the caller
+        says which code each row uses (dist_net_t.row_code, or the view of the pixel in a render)."""
         if engine == _abi.ENGINE_TC:
             from . import tc
             try:
@@ -144,22 +150,24 @@ class DecoderPlan(object):
                 if not getattr(self, "tc_unsafe", False):
                     raise
                 engine = _abi.ENGINE_SIMT       # self-check failed (warned once): this call runs on the fp32 engine
-        b0, bl, lat = self.fold(latent, stream)
+        b0, bl, lat = self.fold(latent, stream, n_codes)
         bl_tc = None
         if engine == _abi.ENGINE_TC and bl is not None:
             from . import tc
             bl_tc = bl * tc.S_ACT
-        net = self.c_net(b0, bl, bl_tc, out_index=out_index)
+        net = self.c_net(b0, bl, bl_tc, out_index=out_index, n_codes=n_codes)
         return net, engine, (b0, bl, bl_tc, lat)
 
-    def c_net(self, bias0, biasl, biasl_tc=None, out_index=0):
+    def c_net(self, bias0, biasl, biasl_tc=None, out_index=0, n_codes=1):
         """ctypes dist_net_t for one call; bias0/biasl are the folded biases (or None before folding); `out_index` selects
-        which output of a multi-output network the (single-output) kernels compute."""
+        which output of a multi-output network the (single-output) kernels compute; n_codes > 1: bias0/biasl are per-code
+        tables (dist_net_t.n_codes)."""
         if not (0 <= out_index < self.n_out):
             raise ValueError("out_index %d outside the decoder's %d outputs" % (out_index, self.n_out))
         net = _abi.Net()
         net.n_layers, net.latent_size, net.latent_in, net.use_tanh = self.n_layers, self.latent_size, \
             self.latent_in, self.use_tanh
+        net.n_codes = int(n_codes) if n_codes > 1 else 0
         for l in range(self.n_layers):
             net.K[l], net.N[l] = self.K[l], self.N[l]
             net.Wt[l], net.W[l] = self.Wt[l].data_ptr(), self.W[l].data_ptr()
@@ -189,12 +197,29 @@ class DecoderPlan(object):
                 net.tc_bias[l] = b.data_ptr()
         return net
 
-    def latent_grad(self, acc0, accl):
-        """dL/dlatent from the accumulated pre-activation gradients of layer 0 and the latent_in layer."""
+    def latent_grad(self, acc0, accl, n_codes=1):
+        """dL/dlatent from the accumulated pre-activation gradients of layer 0 and the latent_in layer: (1, L), or (C, L)
+        from the per-code accumulators [C][N] of a call with n_codes = C > 1."""
+        if n_codes > 1:
+            C = int(n_codes)
+            g = acc0[: C * self.N[0]].reshape(C, self.N[0]) @ self.Wz0
+            if self.latent_in >= 0:
+                g = g + accl[: C * self.N[self.latent_in]].reshape(C, self.N[self.latent_in]) @ self.Wzl
+            return g
         g = acc0[: self.N[0]] @ self.Wz0
         if self.latent_in >= 0:
             g = g + accl[: self.N[self.latent_in]] @ self.Wzl
         return g.reshape(1, -1)
+
+    def acc_buffers(self, n_codes=1):
+        """Zeroed accumulators acc0 / accl of a backward call: [Np4] (one code, as always) or [n_codes][N]."""
+        if n_codes > 1:
+            n0, nl = n_codes * self.N[0], (n_codes * self.N[self.latent_in] if self.latent_in >= 0 else 0)
+        else:
+            n0, nl = self.bias[0].numel(), (self.bias[self.latent_in].numel() if self.latent_in >= 0 else 0)
+        acc0 = torch.zeros(n0, device=self.device, dtype=torch.float32)
+        accl = torch.zeros(nl, device=self.device, dtype=torch.float32) if self.latent_in >= 0 else None
+        return acc0, accl
 
 
 _PLANS = {}

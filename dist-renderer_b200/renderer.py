@@ -50,7 +50,8 @@ class _RenderDepthFn(torch.autograd.Function):
         dev = ren.device
         P, B = ren.P, ren.buffer_size
         engine = resolve_engine(plan, opts["engine"])
-        net, engine, _keep = plan.net_for(latent, engine, st)
+        n_codes = ren._n_codes(latent)     # > 1: view v is rendered with latent[v]
+        net, engine, _keep = plan.net_for(latent, engine, st, n_codes=n_codes)
         Rd = R.detach().float().contiguous()
         if Rd.shape != ((3, 3) if ren.n_views == 1 and R.dim() == 2 else (ren.n_views, 3, 3)):
             raise ValueError("R must be (3,3), or (n_views,3,3) on a multi-view renderer")
@@ -73,7 +74,8 @@ class _RenderDepthFn(torch.autograd.Function):
             "flags": torch.empty(P, device=dev, dtype=torch.uint8), "nreal": torch.empty(P, device=dev, dtype=torch.int32),
             "top_sdf": torch.empty(B, P, **f32), "top_pt": torch.empty(B, 3, P, **f32),
             "top_zafter": torch.empty(B, P, **f32), "top_zgen": torch.empty(B, P, **f32),
-            "sdf_origin": torch.empty(1, **f32), "dist": torch.empty(P, **f32),
+            # sdf at the origin: one per view (the views' own codes when each view has one)
+            "sdf_origin": torch.empty(ren.n_views, **f32), "dist": torch.empty(P, **f32),
             "top_lvl": torch.empty(B, P, device=dev, dtype=torch.uint8),
         }
         scr = ren._scratch(pyramid=pyr)
@@ -99,7 +101,7 @@ class _RenderDepthFn(torch.autograd.Function):
         _abi.check(lib.dist_render_depth_fwd(net, engine, cam, mp, ws, _abi.ptr(Zdepth), _abi.ptr(mask),
                                              _abi.ptr(min_sdf), _abi.ptr(ren.rows_evaluated), st))
         ren._last_counts = scr["view_stat"]
-        ctx.ren, ctx.opts, ctx.engine, ctx.mp, ctx.mask_cap = ren, opts, engine, mp, mask_cap
+        ctx.ren, ctx.opts, ctx.engine, ctx.mp, ctx.mask_cap, ctx.n_codes = ren, opts, engine, mp, mask_cap, n_codes
         ctx.saved = saved
         ctx.save_for_backward(latent, Rd, T.detach().float())
         hit = saved["flags"].bitwise_and(1).bool()
@@ -118,7 +120,7 @@ class _RenderDepthFn(torch.autograd.Function):
         latent, Rd, Td = ctx.saved_tensors
         ren, opts, lib, st = ctx.ren, ctx.opts, _abi.lib(), _stream(ctx.ren.device)
         plan, dev, P, B = ren.plan, ren.device, ren.P, ren.buffer_size
-        net, eng_b, _keep = plan.net_for(latent, ctx.engine, st)
+        net, eng_b, _keep = plan.net_for(latent, ctx.engine, st, n_codes=ctx.n_codes)
         cam_pos = ren.get_camera_location(Rd, Td).contiguous()
         cam = ren._c_camera(Rd, cam_pos, opts["use_transform"])
         V, Pv = ren.n_views, ren.Pv
@@ -135,8 +137,7 @@ class _RenderDepthFn(torch.autograd.Function):
         gM = gM.contiguous().float() if (gM is not None and opts["want_mask_grad"]) else None
         want_cam = opts["cam_levels"] != 0 and (ctx.needs_input_grad[1] or ctx.needs_input_grad[2])
         f32 = dict(device=dev, dtype=torch.float32)
-        acc0 = torch.zeros(plan.bias[0].numel(), **f32)
-        accl = torch.zeros(plan.bias[plan.latent_in].numel(), **f32) if plan.latent_in >= 0 else None
+        acc0, accl = plan.acc_buffers(ctx.n_codes)
         d_cam = torch.zeros(V, 3, **f32) if want_cam else None
         d_ray = torch.zeros(3, P, **f32) if want_cam else None
         n_coarse = V * sum(g[0].shape[1] for g in ren._coarse_homo()) if (want_cam and pyr) else 0
@@ -149,7 +150,7 @@ class _RenderDepthFn(torch.autograd.Function):
                                                  _abi.ptr(d_ray_c), _abi.ptr(s_row), _abi.ptr(s_pts), _abi.ptr(s_coef), None,
                                                  _abi.ptr(s_dpts), _abi.ptr(s_cnt), _abi.ptr(ren.rows_grad), st))
             if ctx.needs_input_grad[0] and latent is not None:
-                g_lat = plan.latent_grad(acc0, accl).reshape(latent.shape).to(latent.dtype)
+                g_lat = plan.latent_grad(acc0, accl, ctx.n_codes).reshape(latent.shape).to(latent.dtype)
             if want_cam:
                 with torch.enable_grad():
                     Rg, Tg = Rd.clone().requires_grad_(True), Td.clone().requires_grad_(True)
@@ -422,6 +423,12 @@ class SDFRenderer(object):
         if int(stat[:, 0].min()) == 0:   # view_stat[v][0]: rays of view v alive at step 0
             raise ValueError('No valid depth.')
 
+    def _n_codes(self, latent):
+        """Latent codes of one call: n_views when a multi-view call gets one code per view (latent (V, L)), else 1."""
+        if self.n_views > 1 and torch.is_tensor(latent) and latent.dim() == 2 and latent.shape[0] == self.n_views:
+            return self.n_views
+        return 1
+
     def reset_row_counter(self):
         self.rows_evaluated.zero_()
         self.rows_grad.zero_()
@@ -519,7 +526,10 @@ class SDFRenderer(object):
                 pts = cam_rays[v, :, idx - v * self.Pv].t() * Zdepth.detach()[idx][None, :] + cam_pos[v].t()
             if use_transform:
                 pts = self.inv_transform_points(pts)
-            o = decode_sdf(self.decoder, latent, pts.t(), clamp_dist=None, engine=self.engine).squeeze(-1)
+            # one code per view: each hit row is decoded with its view's code
+            index = v if (v is not None and self._n_codes(latent) > 1) else None
+            o = decode_sdf(self.decoder, latent, pts.t(), clamp_dist=None, engine=self.engine,
+                           latent_index=index).squeeze(-1)
 
             def dchain(x):     # d sdf / d pre-activation as a function of the sdf value (deep_sdf_decoder.py:99-110)
                 if self.plan.use_tanh:
@@ -534,7 +544,7 @@ class SDFRenderer(object):
         plan = self.plan
         plan.refresh()
         engine = resolve_engine(plan, self.engine)
-        net, engine, _keep = plan.net_for(latent, engine, st)
+        net, engine, _keep = plan.net_for(latent, engine, st, n_codes=self._n_codes(latent))
         Rd = R.detach().float().contiguous()
         cam_pos = self.get_camera_location(Rd, T.detach().float()).contiguous()
         cam = self._c_camera(Rd, cam_pos, use_transform)
@@ -633,8 +643,14 @@ class SDFRenderer(object):
         return slots[:n]
 
     def render_views(self, latent, Rs, Ts, fused=True, n_streams=1, **kw):
-        """``render()`` of V camera poses of one shape, batched: returns the outputs of ``render`` stacked along a
-        new leading view axis -- (depth[V,h,w], normal[V,h,w,3], mask[V,h,w] uint8, min_abs_query[V,h,w]).
+        """``render()`` of V camera poses, batched: returns the outputs of ``render`` stacked along a new leading view
+        axis -- (depth[V,h,w], normal[V,h,w,3], mask[V,h,w] uint8, min_abs_query[V,h,w]).
+
+        ``latent``: one code shared by every view, (1, L) or (L,), or one code per view, (V, L) -- view v is then
+        rendered with ``latent[v]``, exactly as ``render(latent[v], Rs[v], Ts[v])`` renders it, and the gradient reaches
+        ``latent`` as (V, L).  So S shapes (or shapes x poses, ``render_views(codes[shape_of_view], Rs, Ts)``) march
+        together and pay the per-step cost of the march tail once.  (An extension: the reference renders one code per
+        call.)
 
         The multi-view callers of the reference (`optimize_multi.py:62-80`, `renderer_warp.py:108-109`) render their
         views one after the other and synchronise with the host several times per march step.
@@ -651,6 +667,12 @@ class SDFRenderer(object):
         V = len(Rs)
         if V == 0 or len(Ts) != V:
             raise ValueError("render_views needs V >= 1 rotations and as many translations")
+        per_view = False
+        if torch.is_tensor(latent) and latent.dim() == 2 and latent.shape[0] != 1:
+            if latent.shape[0] != V:
+                raise ValueError("latent must be (1, L), (L,) or one code per view (%d, L); got %s"
+                                 % (V, tuple(latent.shape)))
+            per_view = True
         if fused and kw.get("num_forward_sampling", 0) == 0:
             R = Rs if torch.is_tensor(Rs) else torch.stack(list(Rs), 0)
             T = Ts if torch.is_tensor(Ts) else torch.stack(list(Ts), 0)
@@ -659,7 +681,8 @@ class SDFRenderer(object):
         # lazily built caches are created on this stream before any view stream can touch them
         _ = self.calib_map, self._coarse_homo()
         self.plan.refresh()
-        self.plan.net_for(latent, resolve_engine(self.plan, self.engine), main.cuda_stream)  # one-time engine preparation
+        self.plan.net_for(latent[:1] if per_view else latent, resolve_engine(self.plan, self.engine),
+                          main.cuda_stream)  # one-time engine preparation
         n_streams = max(1, min(int(n_streams), V))
         slots = self._view_slots(n_streams)
         side = n_streams > 1
@@ -671,7 +694,7 @@ class SDFRenderer(object):
         for v in range(V):
             st, child = slots[v % n_streams]
             with torch.cuda.stream(st if side else main):
-                o = child.render(latent, Rs[v], Ts[v], check_empty=False, **kw)
+                o = child.render(latent[v] if per_view else latent, Rs[v], Ts[v], check_empty=False, **kw)
                 n_valid[v:v + 1].copy_(child._last_counts[:, 0])
             outs.append(o)
         if side:

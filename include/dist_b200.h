@@ -72,6 +72,14 @@ typedef struct dist_net {
   const float* tc_scale;      /* HOST array: 1/sW per tensor-core layer (forward layers, then the transposed chain) */
   int64_t tc_blob_bytes;
   const float* tc_bias[DIST_MAX_LAYERS]; /* biases in the engine's scaled activation units (bias * 32), per net layer */
+  /* Several latent codes in one call (0 or 1: one code, the layout above).  No counterpart in the reference, which decodes
+   * one code per call.  With n_codes > 1, bias[0], bias[latent_in] and tc_bias[latent_in] point to per-code tables
+   * [n_codes][Np4] (written by dist_fold_latent from latent [n_codes][latent_size]), and the acc0 / accl accumulators of the
+   * backward entry points are [n_codes][N] (N = N[0] / N[latent_in]).  Which code a decoder row uses: */
+  int32_t n_codes;
+  const int32_t* row_code;    /* dist_decoder_*: device [n] code of row i, in [0, n_codes).  Ignored by dist_render_*, where
+                                 the code of a row is the view of its pixel: n_codes must then equal dist_camera_t.n_views
+                                 (DIST_E_INVALID otherwise), view v being rendered with code v */
 } dist_net_t;
 
 /* Camera + image description for one render (renderer.py:13-59,180-200). */
@@ -151,7 +159,8 @@ typedef struct dist_workspace {
   float* pts;        /* [2][2*SEG][3] query points, ping-pong by step parity */
   float* sdf;        /* [2*SEG] decoder outputs of the current step */
   int32_t* counts;   /* [2*(march_step + 2)] active rays per step and segment (8-byte aligned: a step's pair advances with one 64-bit atomic); zeroed by dist_render_depth_fwd */
-  float* sdf_origin; /* [1] sdf at the origin (filler samples, renderer.py:539-540) */
+  float* sdf_origin; /* [1] sdf at the origin (filler samples, renderer.py:539-540); [n_views] when dist_net_t.n_codes > 1
+                        (one origin query per view, with that view's code) */
   float* entry0;     /* [P] true unit-sphere entry depth; == entry except in DIST_MARCH_PYRAMID, where `entry` holds the
                         depth the full-resolution march starts from (inherited from the 1/2-resolution parent ray) */
   uint8_t* top_lvl;  /* [B][P] bits 0-1: pyramid level the sample was taken at (0 = this ray; 1, 2 = parent / grandparent
@@ -212,7 +221,9 @@ int dist_device_supports_tc(int device);
 /* ---- decoder (decoder_utils.py:53-92, deep_sdf_decoder.py:80-111) ---- */
 
 /* Per-render folded biases: out0[n] = b0[n] + Wz0[n,:].latent ; outl likewise for the latent_in layer.
- * Replaces the latent.expand + torch.cat of decoder_utils.py:61-62 and deep_sdf_decoder.py:92-93. */
+ * Replaces the latent.expand + torch.cat of decoder_utils.py:61-62 and deep_sdf_decoder.py:92-93.
+ * net->n_codes > 1: latent is [n_codes][latent_size], out0 / outl are [n_codes][Np4], row c computed exactly as a
+ * single-code call on latent[c] computes it. */
 int dist_fold_latent(const dist_net_t* net, const float* latent, float* out0, float* outl, void* stream);
 
 /* sdf[i] = decoder(latent, points[i]) for i < n (n read from *n_dev when n_dev != NULL, else n_host).
